@@ -2,6 +2,7 @@
 """bench.py -- the driver's benchmark contract for the anti-aliased resize hot path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config cfg2|cfg3|cfg4] [--no-sub]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic images.  The headline workload
 (BASELINE.json configs[1], "cfg2") is fp32 [256,3,1080,1920] channels_last -> (224,224) bilinear
@@ -25,6 +26,11 @@ Prints ONE JSON line on rank 0:
 
 --impl reference times only the reference's CPU implementation (all host threads) and prints the
 same line with "impl": "reference".
+
+--dump-outputs DIR writes, on rank 0, what the timed path returned in its last step as DIR/<name>.npy (NCHW,
+float32): "output" for a forward config, "grad_input" for cfg4.  Inputs are seeded, so two builds run with the
+same arguments can be compared output for output.  An output above DUMP_BYTES keeps a fixed, seeded sample of
+its images (the line's "dump" object says which).
 """
 import argparse
 import json
@@ -50,6 +56,7 @@ CONFIGS = {
                  workload="cfg4: backward of bilinear antialias [64,3,512,512] -> (128,128): grad_out [64,3,128,128] -> grad_in"),
 }
 METRIC = "Mpix/s (input+output pixels), AA bilinear/bicubic resize, and fraction of HBM peak"
+DUMP_BYTES = 32 << 20
 
 
 def mpix(cfg, n_images=None):
@@ -163,6 +170,22 @@ def make_inputs(cfg, dev, torch, n_images=None):
     if cfg["cl"]:
         x = x.contiguous(memory_format=torch.channels_last)
     return x
+
+
+def dump_output(dirname, name, t):
+    """Writes the [N,C,H,W] result `t` as dirname/<name>.npy; above DUMP_BYTES only a seeded sample of its images. -> dict"""
+    import numpy as np
+    import torch
+    if t.dtype not in (torch.float32, torch.float64):
+        t = t.float()
+    n = t.shape[0]
+    keep = min(n, max(1, DUMP_BYTES // (t[:1].numel() * t.element_size())))
+    images = np.arange(n) if keep == n else np.sort(np.random.default_rng(0).permutation(n)[:keep])
+    a = np.ascontiguousarray(t[torch.from_numpy(images).to(t.device)].cpu().numpy())
+    os.makedirs(dirname, exist_ok=True)
+    path = os.path.join(dirname, name + ".npy")
+    np.save(path, a)
+    return {"file": path, "shape": list(a.shape), "dtype": str(a.dtype), "images": images.tolist() if keep < n else "all"}
 
 
 def cpu_reference_rate(cfg, seconds, torch, threads=None):
@@ -479,7 +502,12 @@ def main():
     ap.add_argument("--no-sub", action="store_true", help="skip the sub-measurements (cfg1/3/4/5, strong scaling)")
     ap.add_argument("--sweep-quick", action="store_true", help="cfg5: every 7th point only")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's result under DIR as .npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU path's result; --impl reference times a CPU sample of other images")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     cfg = dict(CONFIGS[args.config])
     if args.images:
@@ -537,6 +565,9 @@ def main():
     capi.check_device(local_rank)
     total_ms_max = reduce_max(torch, dist, world, dev, total_ms)
     clocks = sampler.stop() if rank == 0 else None
+    dump = None
+    if args.dump_outputs and rank == 0:
+        dump = dump_output(args.dump_outputs, "output" if cfg["kind"] == "forward" else "grad_input", out)
 
     # ---- e2e: host buffers through the C ABI, copies inside the timed region, with the copy ceiling beside it
     e2e = None
@@ -599,6 +630,8 @@ def main():
         }
         if e2e:
             line["e2e"] = e2e
+        if dump:
+            line["dump"] = dump
         if sub is not None:
             line["sub"] = sub
         if world == 1 and not args.no_cpu_baseline:

@@ -3,9 +3,10 @@ must be issued before the first FFMA2 that consumes them (ptxas sometimes sinks 
 arithmetic when registers get tight, which serialises the HBM requests -- measured -15 % on cfg2).
 usage: python scripts/sass_lint.py [lib.so]   -> prints, per aa_stream_kernel instantiation, the longest run of
 128/64-bit LDGs that precedes an FFMA2 and flags the ones where that run is shorter than U."""
-import re, subprocess, sys, os
+import re, shutil, subprocess, sys, os
 lib = sys.argv[1] if len(sys.argv) > 1 else os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "interpolate_antialiasing_b200", "_build", "libaa_resize_b200.so")
-out = subprocess.run(["cuobjdump", "-sass", lib], capture_output=True, text=True).stdout
+cuobjdump = shutil.which("cuobjdump") or os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "bin", "cuobjdump")
+out = subprocess.run([cuobjdump, "-sass", lib], capture_output=True, text=True, check=True).stdout
 cur, funcs = None, {}
 for line in out.splitlines():
     m = re.search(r"Function : (\S+)", line)

@@ -17,7 +17,23 @@ def pytest_configure(config):
 
 @pytest.fixture(scope="session")
 def golden():
-    return np.load(os.path.join(GOLDEN_DIR, "golden_v1.npz"))
+    """The stored golden vectors (see tests/golden/make_golden.py).  The seeded inputs of the small cases are not
+    stored: they are drawn again here in the generator's order and must match the sha256 recorded with them."""
+    import hashlib
+    import torch
+    g = {}
+    for name in ("golden_v1.npz", "golden_v1_fp64.npz", "reference_checks_v1.npz"):
+        with np.load(os.path.join(GOLDEN_DIR, name)) as z:
+            g.update({k: z[k] for k in z.files})
+    gen = torch.Generator().manual_seed(1234)
+    for i in range(int(g["n_cases"])):
+        shape, dt = tuple(int(v) for v in g[f"case{i}_shape"]), getattr(torch, str(g[f"case{i}_dtype"]))
+        osize = tuple(int(v) for v in g[f"case{i}_osize"])
+        for key, shp, scale in (("x", shape, 255), ("gout", shape[:2] + osize, 1)):
+            a = (torch.rand(shp, generator=gen, dtype=dt) * scale).numpy()
+            assert hashlib.sha256(a.tobytes()).hexdigest() == str(g[f"case{i}_{key}_sha256"]), (i, key)
+            g[f"case{i}_{key}"] = a
+    return g
 
 
 @pytest.fixture(scope="session")

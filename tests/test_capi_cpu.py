@@ -143,9 +143,10 @@ def test_sass_of_the_built_kernels():
     that follows every fast float launch exists and waits on its programmatic dependency (ACQBULK = griddepcontrol.wait; the float
     tile kernels trigger it with PREEXIT = griddepcontrol.launch_dependents);
     the headline streaming instantiation keeps everything in registers (no local-memory loads or stores)."""
-    import subprocess
+    import shutil, subprocess
     from interpolate_antialiasing_b200 import capi
-    out = subprocess.run(["cuobjdump", "-sass", capi.LIB], capture_output=True, text=True, timeout=600).stdout
+    cuobjdump = shutil.which("cuobjdump") or os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "bin", "cuobjdump")
+    out = subprocess.run([cuobjdump, "-sass", capi.LIB], capture_output=True, text=True, timeout=600, check=True).stdout
     funcs, cur = {}, None
     for line in out.splitlines():
         m = re.search(r"Function : (\S+)", line)
