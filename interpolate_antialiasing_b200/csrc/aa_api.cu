@@ -207,6 +207,22 @@ int forward_impl(const aa_tensor_desc* in, const aa_tensor_desc* out, int filter
     lout.planes = out->n; lout.Cp = 1; lout.Ci = (int)out->c; lout.stride_n = out->stride_n; lout.stride_p = 0;
     lout.stride_h = (out->h == 1) ? out->w : out->stride_h;
   }
+  if (epi.norm && !in_cl && in->c > 1) {
+    // the kernels take the channel of scale[c] / bias[c] from the interleaved column (channels_last); in a channels_first
+    // tensor every plane would get channel 0's.  One call per channel plane, its own scale / bias in slot 0.
+    auto es = [](int dt) { return (int64_t)(dt == AA_U8 ? 1 : (dt == AA_F16 || dt == AA_BF16) ? 2 : (dt == AA_F32 ? 4 : 8)); };
+    for (int64_t c = 0; c < in->c; c++) {
+      aa_tensor_desc di = *in, dd = *out;
+      di.c = dd.c = 1;
+      di.data = (char*)in->data + c * in->stride_c * es(in->dtype);
+      dd.data = (char*)out->data + c * out->stride_c * es(out->dtype);
+      aa_epilogue e1 = *ex;
+      e1.scale[0] = ex->scale[c];
+      e1.bias[0] = ex->bias[c];
+      if ((rc = forward_impl(&di, &dd, filter, align, flags, stream, &e1, sc)) != AA_OK) return rc;
+    }
+    return AA_OK;
+  }
   DeviceGuard g(in->device);
   if (!g.ok) return cuda_fail(g.err, "cudaSetDevice");
   std::shared_ptr<AxisTables> th, tw;

@@ -13,7 +13,7 @@ rnd = random.Random(seed)
 g = torch.Generator().manual_seed(seed)
 dev = torch.device("cuda", 0)
 t0 = time.time()
-n = fails = 0
+n = fails = n_af = 0  # n_af: fast-path results compared bit for bit with their FLAG_ASSUME_FINITE run
 paths = {"auto": capi.FLAG_AUTO, "stream": capi.FLAG_FORCE_STREAM, "tma": capi.FLAG_FORCE_STREAM | capi.FLAG_STREAM_TMA,
          "general": capi.FLAG_FORCE_GENERAL}
 stats = {k: 0 for k in paths}
@@ -66,6 +66,16 @@ while time.time() - t0 < budget:
             print("ERROR", pname, (N, C, H, W), (oH, oW), mode, align, cl, dt, e); fails += 1; continue
         got = y.cpu().numpy()
         n += 1; stats[pname] += 1
+        if dt == torch.float32 and not nonfinite and pname != "general":
+            # the drain kernel behind the fast float kernels recomputes whatever stored a NaN/Inf, so a stale NaN read from
+            # shared memory would be repaired there: without it (FLAG_ASSUME_FINITE) the result must be the same bits
+            poison_smem()
+            ya = capi.resize_forward(xc, (oH, oW), mode, align, fl | capi.FLAG_ASSUME_FINITE)
+            torch.cuda.synchronize()
+            n_af += 1
+            if not torch.equal(ya, y):
+                fails += 1
+                print("ASSUME_FINITE MISMATCH", pname, (N, C, H, W), (oH, oW), mode, align, cl, int((~torch.isfinite(ya)).sum()))
         if nonfinite:
             wbad = ~np.isfinite(want)
             ok = np.array_equal(~np.isfinite(got), wbad)
@@ -100,6 +110,14 @@ while time.time() - t0 < budget:
         gi = capi.resize_backward(gc, (N, C, H, W), mode, align)
         torch.cuda.synchronize()
         n += 1
+        if dt == torch.float32 and not gnf:
+            poison_smem()
+            gia = capi.resize_backward(gc, (N, C, H, W), mode, align, flags=capi.FLAG_ASSUME_FINITE)
+            torch.cuda.synchronize()
+            n_af += 1
+            if not torch.equal(gia, gi):
+                fails += 1
+                print("BWD ASSUME_FINITE MISMATCH", (N, C, H, W), (oH, oW), mode, align, cl, int((~torch.isfinite(gia)).sum()))
         if gnf:
             gbad = ~np.isfinite(wantg)
             gnp = gi.cpu().numpy()
@@ -109,5 +127,5 @@ while time.time() - t0 < budget:
         elif not np.allclose(gi.cpu().numpy(), wantg, rtol=1e-5, atol=4e-6 if dt == torch.float32 else 1e-11):
             fails += 1
             print("BWD MISMATCH", (N, C, H, W), (oH, oW), mode, align, cl, dt, float(np.abs(gi.cpu().numpy() - wantg).max()))
-print(f"fuzz: {n} checks in {time.time() - t0:.0f}s, {fails} failures, per path {stats}")
+print(f"fuzz: {n} checks in {time.time() - t0:.0f}s, {fails} failures, per path {stats}, {n_af} ASSUME_FINITE comparisons")
 sys.exit(1 if fails else 0)

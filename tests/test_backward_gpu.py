@@ -104,33 +104,44 @@ def test_extension_matches_reference_api(cuda, golden):
 
 
 def test_backward_no_out_of_bounds_access(cuda):
+    """NaN margins around grad_output, -12345 margins around grad_input.  The fast adjoint kernels are followed by the
+    drain kernel, which would recompute a region that picked up a canary (aa_redo.cu); so each case runs with
+    FLAG_ASSUME_FINITE (no drain), whose result must be finite and match the oracle, and with the default flags, whose
+    result must be bit-identical to it.  The tile adjoint (backward of a downsampling) and the streaming adjoint
+    (backward of an upsampling, forced) are both covered."""
     from interpolate_antialiasing_b200 import capi
     import ctypes
     g = torch.Generator().manual_seed(6)
-    for shape, osize in [((2, 3, 64, 96), (16, 24)), ((1, 4, 31, 45), (96, 128)), ((2, 1, 57, 64), (19, 20)), ((3, 3, 128, 128), (32, 32))]:
+    pad = 4096
+    for shape, osize, flags in [((2, 3, 64, 96), (16, 24), capi.FLAG_AUTO), ((1, 4, 31, 45), (96, 128), capi.FLAG_AUTO),
+                                ((2, 1, 57, 64), (19, 20), capi.FLAG_AUTO), ((3, 3, 128, 128), (32, 32), capi.FLAG_AUTO),
+                                ((1, 3, 32, 48), (128, 192), capi.FLAG_FORCE_STREAM)]:
         for cl in (False, True):
             for mode in ("linear", "cubic"):
-                pad = 4096
                 gshape = (shape[0], shape[1]) + osize
                 n_in = int(np.prod(gshape)); n_out = int(np.prod(shape))
-                gb = torch.full((n_in + 2 * pad,), float("nan"), device=cuda)
-                ob = torch.full((n_out + 2 * pad,), -12345.0, device=cuda)
-                if cl:
-                    go = gb[pad:pad + n_in].view(gshape[0], gshape[2], gshape[3], gshape[1]).permute(0, 3, 1, 2)
-                    gi = ob[pad:pad + n_out].view(shape[0], shape[2], shape[3], shape[1]).permute(0, 3, 1, 2)
-                else:
-                    go = gb[pad:pad + n_in].view(gshape)
-                    gi = ob[pad:pad + n_out].view(shape)
                 src = torch.rand(gshape, generator=g)
-                go.copy_(src)
-                dg, di = capi.desc(go), capi.desc(gi)
-                capi.check(capi.lib().aa_resize_backward(ctypes.byref(dg), ctypes.byref(di), capi.FILTERS[mode], 0, 0,
-                                                          ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)))
-                torch.cuda.synchronize()
-                assert torch.isfinite(gi).all(), (shape, osize, cl, mode)
-                assert (ob[:pad] == -12345.0).all() and (ob[pad + n_out:] == -12345.0).all()
+                res = []
+                for fl in (flags | capi.FLAG_ASSUME_FINITE, flags):
+                    gb = torch.full((n_in + 2 * pad,), float("nan"), device=cuda)
+                    ob = torch.full((n_out + 2 * pad,), -12345.0, device=cuda)
+                    if cl:
+                        go = gb[pad:pad + n_in].view(gshape[0], gshape[2], gshape[3], gshape[1]).permute(0, 3, 1, 2)
+                        gi = ob[pad:pad + n_out].view(shape[0], shape[2], shape[3], shape[1]).permute(0, 3, 1, 2)
+                    else:
+                        go = gb[pad:pad + n_in].view(gshape)
+                        gi = ob[pad:pad + n_out].view(shape)
+                    go.copy_(src)
+                    dg, di = capi.desc(go), capi.desc(gi)
+                    capi.check(capi.lib().aa_resize_backward(ctypes.byref(dg), ctypes.byref(di), capi.FILTERS[mode], 0, fl,
+                                                              ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)))
+                    torch.cuda.synchronize()
+                    assert (ob[:pad] == -12345.0).all() and (ob[pad + n_out:] == -12345.0).all()
+                    res.append(gi.clone())
+                assert torch.isfinite(res[0]).all(), (shape, osize, cl, mode, "read outside grad_output")
                 want = O.backward_adjoint(src.numpy(), shape, mode, False)
-                np.testing.assert_allclose(gi.cpu().numpy(), want, rtol=1e-5, atol=4e-6)
+                np.testing.assert_allclose(res[0].cpu().numpy(), want, rtol=1e-5, atol=4e-6)
+                assert torch.equal(res[1], res[0]), (shape, osize, cl, mode, "the drain repaired the result")
 
 
 def test_custom_op_compile_and_autograd(cuda):
@@ -187,7 +198,8 @@ def test_backward_with_uncovered_rows_and_columns(cuda):
     """align_corners with a 1-pixel output axis (scale 0: only input index 0 contributes) and the box filter leave
     grad_input rows / columns that NO grad_output element reaches: empty adjoint windows.  Their gathers must read
     initialised memory only (found by the fuzz: a zero weight times stale NaNs in shared memory).  Shared memory is
-    pre-loaded with NaNs by resizing an all-NaN tensor through the same kernels right before every case."""
+    pre-loaded with NaNs by resizing an all-NaN tensor through the same kernels right before every case, and the case
+    runs once with FLAG_ASSUME_FINITE: without the drain kernel behind it, a stale NaN that was read stays visible."""
     from interpolate_antialiasing_b200 import capi
     g = torch.Generator().manual_seed(29)
     poison_f = torch.full((2, 5, 160, 64), float("nan"), device=cuda)
@@ -202,10 +214,10 @@ def test_backward_with_uncovered_rows_and_columns(cuda):
                 gc = go.to(cuda)
                 if cl:
                     gc = gc.contiguous(memory_format=torch.channels_last)
-                for _ in range(2):
+                for flags in (capi.FLAG_ASSUME_FINITE, capi.FLAG_AUTO):
                     capi.resize_forward(poison_f, (120, 48), mode, False)          # band / tile kernels, NaN patches
                     capi.resize_backward(poison_b, (2, 5, 160, 64), mode, False)   # tile kernel (adjoint), NaN patches
-                    got = capi.resize_backward(gc, shp, mode, True)
+                    got = capi.resize_backward(gc, shp, mode, True, flags=flags)
                     torch.cuda.synchronize()
                     a = got.cpu().numpy()
                     assert np.isfinite(a).all(), (shp, osz, mode, cl)

@@ -271,45 +271,94 @@ def test_edge_cases(cuda):
         capi.resize_forward(torch.rand((1, 3, 8, 16), device=cuda)[:, :, :, ::2], (4, 4), "linear")
 
 
-def _guarded(shape, dtype, device, channels_last, pad=4096, fill=float("nan")):
-    """A tensor of `shape` carved out of a larger buffer whose margins hold canaries."""
-    n = int(np.prod(shape))
-    buf = torch.full((n + 2 * pad,), fill if dtype.is_floating_point else 255, dtype=dtype, device=device)
-    core = buf[pad:pad + n]
+def _guarded(shape, dtype, device, channels_last, fill, pad=4096, crop=None):
+    """A tensor of `shape` carved out of a larger buffer filled with `fill` (the canary).  crop=(r0, c0, dh, dw): the
+    tensor is the view [:, :, r0:r0+H, c0:c0+W] of a parent [N, C, H+dh, W+dw] (padded rows, a base pointer c0 elements
+    past a row start, a batch stride larger than one image), the parent itself inside the guarded buffer."""
     N, C, H, W = shape
-    t = core.view(N, H, W, C).permute(0, 3, 1, 2) if channels_last else core.view(N, C, H, W)
-    return buf, t, pad, n
+    r0, c0, dh, dw = crop or (0, 0, 0, 0)
+    Hp, Wp = H + dh, W + dw
+    n = N * C * Hp * Wp
+    buf = torch.full((n + 2 * pad,), fill, dtype=dtype, device=device)
+    core = buf[pad:pad + n]
+    t = core.view(N, Hp, Wp, C).permute(0, 3, 1, 2) if channels_last else core.view(N, C, Hp, Wp)
+    return buf, t[:, :, r0:r0 + H, c0:c0 + W]
+
+
+def _untouched_outside(buf, view, fill):
+    """Every element of `buf` outside `view` still holds `fill`."""
+    b = buf.clone()
+    b.as_strided(view.shape, view.stride(), view.storage_offset() - buf.storage_offset()).fill_(fill)
+    return bool((b == fill).all())
+
+
+# Input views of the canary test: dense, then crops whose base pointer is 1, 2, 4 and 16 elements past a row start
+# (4/8/16-byte aligned fp32 rows: the streaming kernel's 1-, 2- and 4-wide vectors, TMA with padded rows; for uint8 the
+# 16-byte aligned crop is the only one the tensor-core kernel takes).  Parent widths are multiples of 16 elements.
+def _in_views(W):
+    return [None] + [(3, c0, 5, (-W) % 16 + 32) for c0 in (1, 2, 4, 16)]
 
 
 @pytest.mark.parametrize("flags_name", ["FLAG_AUTO", "FLAG_FORCE_STREAM", "FLAG_FORCE_GENERAL", "TMA"])
 def test_no_out_of_bounds_access(cuda, flags_name):
-    """compute-sanitizer is closed on this pool, so out-of-bounds traffic is caught with canaries: NaN
-    margins around the input poison the output if any kernel reads outside the tensor (even with a zero
-    weight), and the output's margins must stay untouched."""
+    """Out-of-bounds traffic is caught with canaries: NaN margins around
+    a float input poison the output if any kernel reads outside the tensor (even with a zero weight), and the output's
+    margins must stay untouched.  A fast float kernel that stores a NaN/Inf gets the region recomputed tap-exactly by
+    the drain kernel behind it (aa_redo.cu), which would repair exactly such a stray read; so every float case also runs
+    with FLAG_ASSUME_FINITE (no drain): that output must be finite and match the oracle, and the default output must be
+    bit-identical to it (finite data stores nothing non-finite, so the drain of a clean kernel has nothing to do).
+    uint8 inputs run with canary 0 and canary 255: identical outputs mean no outside byte was read with any non-zero
+    weight.  Inputs are dense tensors and cropped views of a larger image; outputs are written through `out=` into a
+    dense tensor or into a view with padded rows and an unaligned base pointer."""
     from interpolate_antialiasing_b200 import capi
     flags = (capi.FLAG_FORCE_STREAM | capi.FLAG_STREAM_TMA) if flags_name == "TMA" else getattr(capi, flags_name)
     g = torch.Generator().manual_seed(5)
     cases = [((2, 3, 64, 96), (16, 24)), ((1, 4, 96, 128), (31, 45)), ((2, 1, 57, 64), (19, 20)), ((1, 3, 40, 48), (80, 96)),
-             ((1, 3, 33, 64), (33, 64)), ((1, 2, 120, 36), (30, 72)), ((3, 3, 128, 128), (32, 32))]
+             ((1, 3, 33, 64), (33, 64)), ((1, 2, 120, 36), (30, 72)), ((3, 3, 128, 128), (32, 32)),
+             ((2, 3, 96, 128), (72, 96)),     # 0.75x: band kernel
+             ((2, 1, 64, 64), (128, 112)),    # upsampling: tile kernel
+             ((2, 3, 24, 160), (72, 80))]     # up in H, down in W: two launches
+    ran = 0
     for shape, osize in cases:
-        for cl in (False, True):
-            for mode in ("linear", "cubic"):
-                for dt in (torch.float32, torch.uint8):
-                    xb, x, _, _ = _guarded(shape, dt, cuda, cl)
-                    src = torch.rand(shape, generator=g) * 255
-                    x.copy_(src.to(dt))
-                    ob, out, pad, n = _guarded((shape[0], shape[1]) + osize, torch.float32, cuda, cl, fill=-12345.0)
-                    try:
-                        capi.resize_forward(x, osize, mode, False, flags, out=out)
-                    except capi.AAError as e:
-                        if "-2" in str(e) and flags != capi.FLAG_AUTO:
-                            continue
-                        raise
-                    torch.cuda.synchronize()
-                    assert torch.isfinite(out).all(), (shape, osize, cl, mode, dt, "read outside the input")
-                    assert (ob[:pad] == -12345.0).all() and (ob[pad + n:] == -12345.0).all(), "wrote outside the output"
-                    want = O.forward(src.to(dt).float().numpy(), osize, mode, False)
-                    _close(out.cpu().numpy(), want)
+        oshape = (shape[0], shape[1]) + osize
+        for mode in ("linear", "cubic"):
+            for dt in (torch.float32, torch.uint8):
+                src = (torch.rand(shape, generator=g) * 255).to(dt)
+                want = O.forward(src.float().numpy(), osize, mode, False)
+                for cl in (False, True):
+                    for crop in _in_views(shape[3]):
+                        ocrop = None if crop is None else (1, 1, 2, 32 - osize[1] % 16)  # base pointer 1 pixel past a row start
+                        runs = [(flags, float("nan")), (flags | capi.FLAG_ASSUME_FINITE, float("nan"))] if dt == torch.float32 else \
+                               [(f, c) for f in ([flags, capi.FLAG_VMMA] if flags == capi.FLAG_AUTO else [flags]) for c in (0, 255)]
+                        outs = {}
+                        for fl, canary in runs:
+                            _, x = _guarded(shape, dt, cuda, cl, canary, crop=crop)
+                            x.copy_(src)
+                            ob, out = _guarded(oshape, torch.float32, cuda, cl, -12345.0, crop=ocrop)
+                            try:
+                                capi.resize_forward(x, osize, mode, False, fl, out=out)
+                            except capi.AAError as e:
+                                if "-2" in str(e) and fl != capi.FLAG_AUTO:
+                                    continue
+                                raise
+                            torch.cuda.synchronize()
+                            assert _untouched_outside(ob, out, -12345.0), (shape, osize, cl, mode, dt, crop, fl, "wrote outside the output")
+                            outs[(fl, str(canary))] = out.clone()
+                        key = (shape, osize, cl, mode, dt, crop)
+                        if dt == torch.float32:
+                            if not outs:
+                                continue
+                            y = outs[(flags | capi.FLAG_ASSUME_FINITE, "nan")]
+                            assert torch.isfinite(y).all(), key + ("read outside the input",)
+                            _close(y.cpu().numpy(), want)
+                            assert torch.equal(outs[(flags, "nan")], y), key + ("the drain repaired the output",)
+                            ran += 1
+                        else:
+                            for fl in {f for f, _ in outs}:
+                                assert torch.equal(outs[(fl, "0")], outs[(fl, "255")]), key + (fl, "read outside the input")
+                                _close(outs[(fl, "0")].cpu().numpy(), want)
+                                ran += 1
+    assert ran > 0
 
 
 def test_cuda_graph_capture_and_replay(cuda):
