@@ -192,6 +192,8 @@ def test_ragged_images_to_fixed_batch(cuda):
     o16, launches = capi.resize_forward_ragged(fimgs, (32, 40), "cubic", out=o16, scale=[1 / 58.0] * 3, bias=[-2.0] * 3)
     torch.cuda.synchronize()
     assert launches == 3
+    from test_epilogue_gpu import affine_ref, assert_rounded, fast_eps, got64, ref_forward
     for i, im in enumerate(fimgs):
-        want = O.forward(im[None].cpu().numpy(), (32, 40), "cubic", False) / 58.0 - 2.0
-        assert np.abs(o16[i:i + 1].float().cpu().numpy() - want).max() < 4e-3
+        base = ref_forward(im[None].cpu().numpy(), (32, 40), "cubic")
+        want = affine_ref(base, [1 / 58.0] * 3, [-2.0] * 3)
+        assert_rounded(got64(o16[i:i + 1]), want, fast_eps(base, want, [1 / 58.0] * 3), "f16", ("ragged fp16", i))

@@ -113,6 +113,7 @@ def test_vmma_batch_slices_and_planes(cuda):
 def test_vmma_decode_adjacent_epilogue(cuda):
     """HWC uint8 -> resize -> normalise -> CHW fp16 (aa_resize_forward_ex) on the tensor-core path."""
     from interpolate_antialiasing_b200 import capi
+    from test_epilogue_gpu import affine_ref, assert_rounded, fast_eps, got64, ref_forward
     g = torch.Generator().manual_seed(12)
     x = torch.randint(0, 256, (2, 3, 480, 640), dtype=torch.uint8, generator=g).to(cuda).contiguous(memory_format=torch.channels_last)
     mean, std = [123.7, 116.3, 103.5], [58.4, 57.1, 57.4]
@@ -122,6 +123,6 @@ def test_vmma_decode_adjacent_epilogue(cuda):
     capi.resize_forward_ex(x, (112, 112), "linear", out, scale, bias, flags=capi.FLAG_VMMA)
     torch.cuda.synchronize()
     capi.check_device(0)
-    want = O.forward(x.float().cpu().numpy(), (112, 112), "linear")
-    want = (want - np.array(mean, np.float32)[None, :, None, None]) / np.array(std, np.float32)[None, :, None, None]
-    assert np.abs(out.float().cpu().numpy() - want).max() < 4e-3
+    base = ref_forward(x.cpu().numpy(), (112, 112), "linear")
+    want = affine_ref(base, scale, bias)
+    assert_rounded(got64(out), want, fast_eps(base, want, scale), "f16", "vmma decode-adjacent fp16")
