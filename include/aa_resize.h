@@ -209,6 +209,32 @@ int aa_resize_forward_ragged(const aa_image_desc* images, int32_t count, int32_t
                              const aa_tensor_desc* out, int filter, int align_corners, uint32_t flags,
                              const aa_epilogue* epilogue, void* cuda_stream, int32_t* launches_out);
 
+/* Batched resized crops: the training-time RandomResizedCrop + RandomHorizontalFlip of an input pipeline, a box per image
+ * resized to one common (oH, oW) in a single launch (torchvision's resized_crop(img, top, left, height, width, size,
+ * antialias=True); not in the reference).  out[i] is the aa_resize_forward_ex result for the view
+ * image_i[top:top+height, left:left+width] (same out dtypes and epilogue, table scale height/oH and width/oW or the
+ * align_corners form), bit for bit the AA_FLAG_FORCE_GENERAL arithmetic; with hflip != 0 output column ox is stored at
+ * oW-1-ox (channels keep their order).  The same image may appear several times in `images` (multi-crop).
+ *   - input u8 or f32, planar (stride_c) or HWC (channels_last != 0), any stride_h; out [count, channels, oH, oW] f32, u8,
+ *     f16 or bf16, channels_first or channels_last (channels_last only for an HWC input); epilogue may be NULL;
+ *   - the weights are computed inside the kernel (no table cache, no allocation, no copy, no synchronisation: capturable
+ *     in a CUDA graph); the crop descriptors travel in the kernel parameters, 512 crops per launch, so a call issues
+ *     ceil(count / 512) launches (*launches_out);
+ *   - only in-window taps inside the boxes are read: NaN/Inf placement is exact with one launch, float input included;
+ *   - AA_ERR_INVALID (message names the crop index) for a box outside its image (top < 0, left < 0, height < 1, width < 1,
+ *     top+height > h, left+width > w), a wrong `out` shape or a null pointer; AA_ERR_UNSUPPORTED for f64 input, the
+ *     path-forcing flags (FORCE_STREAM, STREAM_TMA, STREAM_LDG, VMMA, FORCE_GENERAL) and a window longer than 65 taps
+ *     (interp_size 2*ceil(support)+1 > 65: box/bicubic/bilinear downscales by more than 64x / 16x / 32x along an axis).
+ *     ASSUME_FINITE and STRICT_NONFINITE change nothing.  Every check happens before the first launch.
+ *   - count == 0 is a no-op. */
+typedef struct aa_crop {
+  int64_t top, left, height, width; /* the box in pixels of its image, torchvision's resized_crop order */
+  int32_t hflip;                    /* != 0: flip the resized result horizontally */
+} aa_crop;
+int aa_resize_crops(const aa_image_desc* images, const aa_crop* crops, int32_t count, int32_t dtype, int64_t channels,
+                    int32_t channels_last, const aa_tensor_desc* out, int filter, int align_corners, uint32_t flags,
+                    const aa_epilogue* epilogue, void* cuda_stream, int32_t* launches_out);
+
 /* grad_in = Wh^T * grad_out * Ww : the true adjoint of aa_resize_forward, gather form, no atomics,
  * no zero-fill pass.  Replaces ti_upsample_bilinear2d_backward_cpu,
  * aa_interpolation_backward_impl.h:185-219 (linear_backward), whose body is the NON-antialiased

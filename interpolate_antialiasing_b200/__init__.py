@@ -18,7 +18,7 @@ from . import capi
 from ._build_ext import EXT, EXT_NAME, LIB
 
 __all__ = ["load", "linear_forward", "cubic_forward", "nearest_forward", "linear_backward", "cubic_backward",
-           "nearest_backward", "linear_backward_nonaa", "forward_with_flags", "resize_to_uint8", "decode_resize_normalize", "AAResize", "aa_resize", "capi"]
+           "nearest_backward", "linear_backward_nonaa", "forward_with_flags", "resize_to_uint8", "decode_resize_normalize", "resized_crops", "AAResize", "aa_resize", "capi"]
 
 _ext = None
 
@@ -99,6 +99,42 @@ def decode_resize_normalize(x_hwc_u8, output_size, mean, std, mode="bilinear", o
     scale = [1.0 / (255.0 * s) for s in std]
     bias = [-m / s for m, s in zip(mean, std)]
     return capi.resize_forward_ex(x, output_size, mode, out, scale, bias, align_corners)
+
+
+def resized_crops(images, boxes, size, mode="bilinear", hflip=None, mean=None, std=None, out_dtype=None, align_corners=False):
+    """RandomResizedCrop + RandomHorizontalFlip of a batch in one kernel launch: torchvision's
+    `resized_crop(img, top, left, height, width, size, antialias=True)` per image, with its own box, optionally flipped.
+
+    images: a list of CUDA tensors, all [H,W,C] (HWC uint8 as a decoder emits; C <= 4) or all [C,H,W], uint8 or float32,
+            or one 4-D [N,C,H,W] tensor (contiguous or channels_last).  An image may repeat (several boxes of one image).
+    boxes:  (top, left, height, width) per image, e.g. from torchvision.transforms.RandomResizedCrop.get_params; each box
+            must lie inside its image.
+    hflip:  optional booleans per image.
+    mean/std: the affine map of decode_resize_normalize, (x/255 - mean)/std, fused into the store; the output is float16
+            unless out_dtype says otherwise.  Without them the output is float32, or uint8 rounded to nearest with
+            out_dtype=torch.uint8.
+    Returns a contiguous [N,C,oH,oW] tensor."""
+    import torch
+    if torch.is_tensor(images):
+        assert images.dim() == 4 and images.is_cuda
+        cl = images.is_contiguous(memory_format=torch.channels_last) and not images.is_contiguous()
+        images = [t.permute(1, 2, 0) if cl else t for t in images.unbind(0)]
+    if isinstance(boxes, torch.Tensor):
+        boxes = boxes.tolist()
+    if hflip is not None and isinstance(hflip, torch.Tensor):
+        hflip = hflip.tolist()
+    oH, oW = (int(size), int(size)) if isinstance(size, int) else (int(size[0]), int(size[1]))
+    hwc = capi._is_hwc(images[0])
+    C = images[0].shape[-1] if hwc else images[0].shape[0]
+    scale = bias = None
+    if mean is not None or std is not None:
+        scale = [1.0 / (255.0 * s) for s in std]
+        bias = [-m / s for m, s in zip(mean, std)]
+        out_dtype = out_dtype or torch.float16
+    out = torch.empty((len(images), C, oH, oW), dtype=out_dtype or torch.float32, device=images[0].device)
+    flags = capi.FLAG_ROUND_NEAREST if out.dtype == torch.uint8 else capi.FLAG_AUTO
+    return capi.resize_crops(images, boxes, (oH, oW), mode, out=out, hflip=hflip, scale=scale, bias=bias,
+                             align_corners=align_corners, flags=flags)[0]
 
 
 from .functional import AAResize, aa_resize  # noqa: E402

@@ -19,7 +19,7 @@ FILTERS = {"nearest": BOX, "box": BOX, "bilinear": TRIANGLE, "linear": TRIANGLE,
 
 EXPORTS = [
     "aa_abi_version", "aa_last_error", "aa_interp_size", "aa_host_tables", "aa_build_tables", "aa_build_tables_sf", "aa_warm_tables",
-    "aa_clear_table_cache", "aa_check_device", "aa_debug_counters", "aa_resize_forward", "aa_resize_forward_sf", "aa_resize_backward_sf", "aa_resize_forward_ex", "aa_resize_forward_ragged", "aa_resize_backward",
+    "aa_clear_table_cache", "aa_check_device", "aa_debug_counters", "aa_resize_forward", "aa_resize_forward_sf", "aa_resize_backward_sf", "aa_resize_forward_ex", "aa_resize_forward_ragged", "aa_resize_crops", "aa_resize_backward",
     "aa_resize_backward_nonaa_bilinear", "aa_resize_forward_host", "aa_resize_forward_host_multi", "aa_launch_count",
 ]
 
@@ -43,6 +43,12 @@ class Epilogue(ctypes.Structure):
 class ImageDesc(ctypes.Structure):
     _fields_ = [("data", ctypes.c_void_p), ("h", ctypes.c_int64), ("w", ctypes.c_int64), ("stride_h", ctypes.c_int64),
                 ("stride_c", ctypes.c_int64)]
+
+
+class Crop(ctypes.Structure):
+    """aa_crop: a box (top, left, height, width) in pixels of its image and an optional horizontal flip."""
+    _fields_ = [("top", ctypes.c_int64), ("left", ctypes.c_int64), ("height", ctypes.c_int64), ("width", ctypes.c_int64),
+                ("hflip", ctypes.c_int32)]
 
 
 class Scales(ctypes.Structure):
@@ -78,6 +84,7 @@ def lib():
         L.aa_resize_backward_sf.argtypes = [P(TensorDesc), P(TensorDesc), i32, i32, P(Scales), u32, vp]
         L.aa_resize_forward_ex.argtypes = [P(TensorDesc), P(TensorDesc), i32, i32, u32, P(Epilogue), vp]
         L.aa_resize_forward_ragged.argtypes = [P(ImageDesc), i32, i32, i64, i32, P(TensorDesc), i32, i32, u32, P(Epilogue), vp, P(i32)]
+        L.aa_resize_crops.argtypes = [P(ImageDesc), P(Crop), i32, i32, i64, i32, P(TensorDesc), i32, i32, u32, P(Epilogue), vp, P(i32)]
         L.aa_resize_backward.argtypes = [P(TensorDesc), P(TensorDesc), i32, i32, u32, vp]
         L.aa_resize_backward_nonaa_bilinear.argtypes = [P(TensorDesc), P(TensorDesc), i32, vp]
         L.aa_resize_forward_host.argtypes = [P(TensorDesc), P(TensorDesc), i32, i32, u32]
@@ -192,11 +199,26 @@ def resize_forward_ex(x, output_size, filter, out, scale=None, bias=None, align_
     return out
 
 
+def _is_hwc(t):
+    """A 3-D image is taken as [H, W, C] (what a decoder emits) when its last axis is a dense interleave of at most 4 channels,
+    else as planar [C, H, W]."""
+    return t.dim() == 3 and t.stride(-1) == 1 and t.shape[-1] <= 4 and t.stride(1) == t.shape[-1]
+
+
+def _epilogue(scale, bias):
+    e = Epilogue()
+    e.normalize = 1 if scale is not None else 0
+    for i in range(4):
+        e.scale[i] = float(scale[i]) if scale is not None and i < len(scale) else 1.0
+        e.bias[i] = float(bias[i]) if bias is not None and i < len(bias) else 0.0
+    return e
+
+
 def resize_forward_ragged(images, output_size, filter, out=None, align_corners=False, flags=FLAG_AUTO, scale=None, bias=None):
     """Variable-size images -> one fixed-size batch (aa_resize_forward_ragged).  `images`: list of CUDA tensors, all [C,H_i,W_i]
     (planar) or all [H_i,W_i,C] (HWC, as a decoder emits), same dtype.  Returns (out [N,C,oH,oW], launches)."""
     import torch
-    hwc = images[0].dim() == 3 and images[0].stride(-1) == 1 and images[0].shape[-1] <= 4 and images[0].stride(1) == images[0].shape[-1]
+    hwc = _is_hwc(images[0])
     C = images[0].shape[-1] if hwc else images[0].shape[0]
     oH, oW = int(output_size[0]), int(output_size[1])
     if out is None:
@@ -224,6 +246,44 @@ def resize_forward_ragged(images, output_size, filter, out=None, align_corners=F
                                          int(align_corners), flags, ctypes.byref(e) if e is not None else None, _stream(out),
                                          ctypes.byref(n)))
     return out, n.value
+
+
+def resize_crops(images, boxes, output_size, filter, out=None, hflip=None, scale=None, bias=None, align_corners=False, flags=FLAG_AUTO):
+    """Batched resized crops (aa_resize_crops): out[i] = resize(images[i][top:top+height, left:left+width]) to output_size,
+    flipped horizontally where hflip[i].  `images`: list of CUDA tensors, all [H_i,W_i,C] (HWC) or all [C,H_i,W_i] (planar), same
+    dtype (uint8 or float32); an image may repeat.  `boxes`: (top, left, height, width) per image.  `out` defaults to a
+    contiguous float32 [N,C,oH,oW]; scale/bias (per channel, <= 4) apply v*scale[c] + bias[c] at the store.
+    Returns (out, launches)."""
+    import torch
+    n = len(images)
+    if len(boxes) != n or (hflip is not None and len(hflip) != n):
+        raise ValueError("resize_crops: images, boxes and hflip must have the same length")
+    hwc = bool(n) and _is_hwc(images[0])
+    if n:
+        C = images[0].shape[-1] if hwc else images[0].shape[0]
+    elif out is not None:
+        C = out.shape[1]
+    else:
+        raise ValueError("resize_crops: an empty batch needs `out`")
+    oH, oW = int(output_size[0]), int(output_size[1])
+    if out is None:
+        out = torch.empty((n, C, oH, oW), dtype=torch.float32, device=images[0].device)
+    arr = (ImageDesc * max(n, 1))()
+    crops = (Crop * max(n, 1))()
+    for i, t in enumerate(images):
+        if hwc:
+            arr[i] = ImageDesc(t.data_ptr(), t.shape[0], t.shape[1], t.stride(0), 1)
+        else:
+            arr[i] = ImageDesc(t.data_ptr(), t.shape[1], t.shape[2], t.stride(1), t.stride(0))
+        top, left, h, w = (int(v) for v in boxes[i])
+        crops[i] = Crop(top, left, h, w, int(bool(hflip[i])) if hflip is not None else 0)
+    e = _epilogue(scale, bias)
+    k = ctypes.c_int32(0)
+    dtype = _dtype_code(images[0]) if n else F32
+    do = desc(out)
+    check(lib().aa_resize_crops(arr, crops, n, dtype, C, int(hwc), ctypes.byref(do), _filter(filter), int(align_corners), flags,
+                                ctypes.byref(e), _stream(out), ctypes.byref(k)))
+    return out, k.value
 
 
 def resize_backward(grad_out, input_size, filter, align_corners=False, nonaa=False, flags=FLAG_AUTO, scales=None, out=None):

@@ -451,6 +451,68 @@ int aa_resize_forward_ragged(const aa_image_desc* images, int32_t count, int32_t
   return AA_OK;
 }
 
+int aa_resize_crops(const aa_image_desc* images, const aa_crop* crops, int32_t count, int32_t dtype, int64_t channels,
+                    int32_t channels_last, const aa_tensor_desc* out, int filter, int align_corners, uint32_t flags,
+                    const aa_epilogue* epilogue, void* cuda_stream, int32_t* launches_out) {
+  int rc;
+  if (launches_out) *launches_out = 0;
+  if (count < 0 || (count > 0 && (!images || !crops))) return fail(AA_ERR_INVALID, "aa_resize_crops: null image or crop list");
+  if ((rc = check_desc(out, "output")) != AA_OK) return rc;
+  if ((rc = check_filter(filter)) != AA_OK) return rc;
+  if (dtype == AA_F64) return fail(AA_ERR_UNSUPPORTED, "aa_resize_crops: input dtype must be u8 or f32");
+  if (dtype != AA_U8 && dtype != AA_F32) return fail(AA_ERR_INVALID, "aa_resize_crops: input dtype must be u8 or f32");
+  if (flags & (AA_FLAG_FORCE_STREAM | AA_FLAG_STREAM_TMA | AA_FLAG_STREAM_LDG | AA_FLAG_VMMA | AA_FLAG_FORCE_GENERAL))
+    return fail(AA_ERR_UNSUPPORTED, "aa_resize_crops: has one kernel; the path-forcing flags do not apply");
+  if (channels < 1 || out->n != count || out->c != channels)
+    return fail(AA_ERR_INVALID, "aa_resize_crops: output must be [count, channels, oH, oW]");
+  const int64_t ci = channels_last ? channels : 1;
+  if (out->h >= (1ll << 31) || out->w * ci >= (1ll << 31)) return fail(AA_ERR_UNSUPPORTED, "aa_resize_crops: output plane too large");
+  if (!channels_last && channels > 65535) return fail(AA_ERR_UNSUPPORTED, "aa_resize_crops: more than 65535 planar channels");
+  OutEpi epi;
+  epi.round = (flags & AA_FLAG_ROUND_NEAREST) ? 1 : 0;
+  switch (out->dtype) {
+    case AA_F32: epi.kind = 0; break;
+    case AA_U8: epi.kind = 1; break;
+    case AA_F16: epi.kind = 2; break;
+    case AA_BF16: epi.kind = 3; break;
+    default: return fail(AA_ERR_INVALID, "aa_resize_crops: output dtype must be f32, u8, f16 or bf16");
+  }
+  if (epilogue && epilogue->normalize) {
+    if (channels > 4) return fail(AA_ERR_UNSUPPORTED, "normalisation epilogue: at most 4 channels");
+    epi.norm = 1;
+    for (int i = 0; i < 4; i++) { epi.scale[i] = epilogue->scale[i]; epi.bias[i] = epilogue->bias[i]; }
+  }
+  // out: channels_first, or channels_last for an HWC input (the memory formats aa_resize_forward_ex accepts)
+  Layout lout;
+  bool out_cl = false;
+  if ((rc = classify_layout(*out, channels_last != 0, &lout, &out_cl)) != AA_OK) return rc;
+  if (out_cl && !channels_last && channels > 1)
+    return fail(AA_ERR_UNSUPPORTED, "aa_resize_crops: a planar input needs a channels_first output");
+  for (int32_t i = 0; i < count; i++) {
+    const aa_image_desc& m = images[i];
+    const aa_crop& b = crops[i];
+    const std::string at = "aa_resize_crops: crop " + std::to_string(i);
+    if (!m.data || m.h <= 0 || m.w <= 0) return fail(AA_ERR_INVALID, at + ": image is empty");
+    if (m.stride_h < m.w * ci) return fail(AA_ERR_INVALID, at + ": rows of the image overlap");
+    if (b.top < 0 || b.left < 0 || b.height < 1 || b.width < 1 || b.height > m.h - b.top || b.width > m.w - b.left)
+      return fail(AA_ERR_INVALID, at + ": box (top " + std::to_string(b.top) + ", left " + std::to_string(b.left) + ", height " +
+                                      std::to_string(b.height) + ", width " + std::to_string(b.width) + ") is not inside its " +
+                                      std::to_string(m.h) + "x" + std::to_string(m.w) + " image");
+    if (b.height >= (1ll << 31) || b.width >= (1ll << 31)) return fail(AA_ERR_UNSUPPORTED, at + ": box too large");
+    if (host_interp_size(b.height, out->h, filter, align_corners, AA_F32) > kCropMaxTaps ||
+        host_interp_size(b.width, out->w, filter, align_corners, AA_F32) > kCropMaxTaps)
+      return fail(AA_ERR_UNSUPPORTED, at + ": window longer than " + std::to_string(kCropMaxTaps) + " taps (downscale too large)");
+  }
+  if (count == 0) return AA_OK;
+  DeviceGuard g(out->device);
+  if (!g.ok) return cuda_fail(g.err, "cudaSetDevice");
+  int32_t launches = 0;
+  rc = launch_crops(images, crops, count, dtype, channels, channels_last, out, filter, align_corners ? 1 : 0, epi,
+                    (cudaStream_t)cuda_stream, &launches);
+  if (launches_out) *launches_out = launches;
+  return rc;
+}
+
 static int backward_impl(const aa_tensor_desc* gout, const aa_tensor_desc* gin, int filter, int align_corners, uint32_t flags,
                          void* cuda_stream, const aa_scales* sc) {
   int rc;

@@ -105,6 +105,8 @@ int ensure_vq_tables(AxisTables* t, int oyb_max, int kstep, int max_ksteps, cuda
 int clear_table_cache();
 // Host-only K computation (no device), same arithmetic as the table kernel.
 int host_interp_size(int64_t in, int64_t out, int filter, int align, int dtype, double user_scale = 0.0);
+// The fp32 table scale of an axis without a caller scale factor (area_pixel_compute_scale<float>), as the table kernel gets it.
+float host_scale_f32(int64_t in, int64_t out, int align);
 
 // ---- layout --------------------------------------------------------------------------------
 // Both supported memory formats are expressed as `planes` independent 2-D images whose rows are
@@ -409,6 +411,14 @@ int vmma_check_watchdog(int device);
 int vmma_read_counters(int device, unsigned long long* out, int reset);
 int vmma_warm(AxisTables* th, cudaStream_t stream);  // everything a later launch_vmma would allocate or synchronise for
 void vmma_plan_clear();
+
+// Batched resized crops (aa_crops.cu): arguments validated by aa_resize_crops; ceil(count / kCropsPerLaunch) launches,
+// counted into *launches.  The per-crop descriptors travel in the kernel parameters (48 bytes each).
+constexpr int kCropsPerLaunch = 512;
+constexpr int kCropMaxTaps = 65;  // largest interp_size (2*ceil(support)+1) of a crop axis: shared weight rows
+int launch_crops(const aa_image_desc* images, const aa_crop* crops, int32_t count, int32_t dtype, int64_t channels,
+                 int32_t channels_last, const aa_tensor_desc* out, int filter, int align, const OutEpi& epi, cudaStream_t stream,
+                 int32_t* launches);
 
 int launch_backward_nonaa(const void* gout, void* gin, int dtype, const Layout& lout, const Layout& lin,
                           int64_t oH, int64_t oW, int64_t H, int64_t W, int align, cudaStream_t stream);

@@ -1,0 +1,191 @@
+// aa_crops.cu -- batched resized crops (aa_resize_crops): one box per crop, any box size, one output size, one launch.
+//
+//   out[n, c, oy, ox'] = sum_y sum_x Wh_n[oy, y] * Ww_n[ox, x] * image_n[top_n + y, left_n + x, c],  ox' = hflip ? oW-1-ox : ox
+//
+// Random boxes almost never share a size, so table caches and per-size launch plans do not pay here: every CTA computes
+// the tables of its own tile (xmin, xsize and weights of its output rows and of its tile's pixel columns) into shared
+// memory with aa_window_f32, the same device function as the K1 table kernel, and the per-crop parameters travel in the
+// kernel parameters.  No allocation, no copy, no synchronisation: the call is CUDA-graph capturable as it stands.
+//
+// Arithmetic: the EXACT order of aa_general_kernel -- horizontal pass into shared T rounded to fp32, then the vertical
+// pass with ascending taps, separate multiply and add -- so every output is bit-identical to aa_resize_forward_ex on the
+// crop's view with AA_FLAG_FORCE_GENERAL.  Only the in-window taps inside the box are read, so NaN/Inf land exactly where
+// the reference puts them without the drain kernel behind the fast float paths.
+#include <algorithm>
+
+#include "aa_common.cuh"
+#include "aa_window.cuh"
+
+namespace aa {
+namespace {
+
+constexpr int TW = 64;           // flat output columns per tile
+constexpr int TH = 32;           // output rows per tile
+constexpr int NTY = 4;           // thread rows
+constexpr int RPT = TH / NTY;    // output rows per thread
+constexpr int RC = 32;           // input rows per chunk
+constexpr int HPT = RC / NTY;    // horizontal-pass rows per thread per chunk
+constexpr int KP = kCropMaxTaps; // weight row pitch in shared memory (odd: the columns of a warp hit distinct banks)
+
+// One crop, 48 bytes.  src already points at the box's first element (top, left) of channel 0, offset in 64 bits.
+struct CropDesc {
+  const void* src;
+  int64_t stride_h, stride_c;  // elements; stride_c: between channel planes (planar input)
+  int32_t h, w;                // box size
+  float scale_h, scale_w;      // fp32 table scales of the two axes (h_scale_f32 of box -> output)
+  int16_t kh, kw;              // interp_size of the two axes (<= kCropMaxTaps)
+  int32_t hflip;
+};
+static_assert(sizeof(CropDesc) == 48, "CropDesc layout");
+
+struct CropParams {
+  void* out;
+  OutEpi epi;
+  int64_t out_sn, out_sc, out_sh, out_sw;  // output element strides
+  int64_t first;                           // output slot of c[0]
+  int oH, oW, Ci, filter, tiles_x;
+  CropDesc c[kCropsPerLaunch];
+};
+// sm_100 takes up to 32764 bytes of kernel parameters
+static_assert(sizeof(CropParams) <= 32764, "kCropsPerLaunch too large for the kernel parameter space");
+
+template <typename in_t>
+__device__ __forceinline__ float ld_in(const in_t* p) { return (float)__ldg(p); }
+
+// One CTA: a TH x TW tile of the flat output (pixel columns x interleaved channels) of one plane of one crop.
+template <typename in_t>
+__global__ void __launch_bounds__(TW* NTY) aa_crops_kernel(const __grid_constant__ CropParams P) {
+  __shared__ float Ts[RC][TW + 1];
+  __shared__ float sWh[TH][KP];
+  __shared__ float sWw[TW][KP];
+  __shared__ int32_t sHs[TH], sHn[TH], sWs[TW], sWn[TW];
+  const CropDesc& D = P.c[blockIdx.z];
+  const int tid = threadIdx.x, tx = tid % TW, ty = tid / TW;
+  const int Ci = P.Ci;
+  const int owf = P.oW * Ci;
+  const int tile_x = (int)(blockIdx.x % (unsigned)P.tiles_x), tile_y = (int)(blockIdx.x / (unsigned)P.tiles_x);
+  const int plane = blockIdx.y;  // channel plane of a planar input; 0 for an interleaved (HWC) one
+  const int oy0 = tile_y * TH, of0 = tile_x * TW;
+  const int nrows = min(TH, P.oH - oy0);
+  const int px0 = of0 / Ci;
+  const int npx = (min(of0 + TW, owf) - 1) / Ci - px0 + 1;
+
+  // ---- the tile's tables, K1 arithmetic
+  for (int k = tid; k < TH + TW; k += TW * NTY) {
+    if (k < TH) {
+      if (k < nrows) aa_window_f32(D.h, P.filter, D.scale_h, D.kh, oy0 + k, &sHs[k], &sHn[k], sWh[k]);
+    } else if (k - TH < npx) {
+      const int j = k - TH;
+      aa_window_f32(D.w, P.filter, D.scale_w, D.kw, px0 + j, &sWs[j], &sWn[j], sWw[j]);
+    }
+  }
+  __syncthreads();
+
+  const int of = of0 + tx;
+  const bool col_ok = of < owf;
+  int px = px0, c = 0, wst = 0, wsz = 0;
+  if (col_ok) {
+    px = of / Ci;
+    c = of - px * Ci;
+    wst = sWs[px - px0];
+    wsz = sWn[px - px0];
+  }
+  const float* wrow = sWw[px - px0];
+  const in_t* icol = (const in_t*)D.src + plane * D.stride_c + (int64_t)wst * Ci + c;
+  int hst[RPT], hsz[RPT];
+  float acc[RPT];
+#pragma unroll
+  for (int r = 0; r < RPT; r++) {
+    const int oyl = ty + r * NTY;
+    acc[r] = 0.f;
+    if (oyl < nrows) { hst[r] = sHs[oyl]; hsz[r] = sHn[oyl]; }
+    else { hst[r] = 0; hsz[r] = 0; }
+  }
+  // box rows the tile needs (window starts and ends are non-decreasing in the output index)
+  const int row_begin = sHs[0];
+  const int row_end = sHs[nrows - 1] + sHn[nrows - 1];
+
+  for (int r0 = row_begin; r0 < row_end; r0 += RC) {
+    // ---- horizontal pass of box rows [r0, r0+RC) for this tile's columns -> Ts (ascending taps, multiply then add)
+    float t[HPT];
+#pragma unroll
+    for (int i = 0; i < HPT; i++) t[i] = 0.f;
+    if (col_ok) {
+      for (int k = 0; k < wsz; k++) {
+        const float wk = wrow[k];
+        const in_t* src = icol + (int64_t)k * Ci;
+#pragma unroll
+        for (int i = 0; i < HPT; i++) {
+          const int row = r0 + ty + i * NTY;
+          if (row < row_end) t[i] = __fadd_rn(t[i], __fmul_rn(ld_in(src + (int64_t)row * D.stride_h), wk));
+        }
+      }
+    }
+#pragma unroll
+    for (int i = 0; i < HPT; i++) Ts[ty + i * NTY][tx] = t[i];
+    __syncthreads();
+    // ---- vertical accumulation over this chunk, ascending rows
+#pragma unroll
+    for (int r = 0; r < RPT; r++) {
+      const int a = hst[r] > r0 ? hst[r] : r0;
+      const int e = min(hst[r] + hsz[r], r0 + RC);
+      const float* hrow = sWh[ty + r * NTY];
+      for (int row = a; row < e; row++) acc[r] = __fadd_rn(acc[r], __fmul_rn(Ts[row - r0][tx], hrow[row - hst[r]]));
+    }
+    __syncthreads();
+  }
+  if (col_ok) {
+    const int ch = plane + c;  // one of the two is 0
+    const int oxs = D.hflip ? P.oW - 1 - px : px;
+    const int64_t base = (P.first + blockIdx.z) * P.out_sn + ch * P.out_sc + oxs * P.out_sw;
+#pragma unroll
+    for (int r = 0; r < RPT; r++) {
+      const int oyl = ty + r * NTY;
+      if (oyl < nrows) aa_store<true>(P.out, base + (int64_t)(oy0 + oyl) * P.out_sh, acc[r], ch, P.epi);
+    }
+  }
+}
+
+}  // namespace
+
+int launch_crops(const aa_image_desc* images, const aa_crop* crops, int32_t count, int32_t dtype, int64_t channels,
+                 int32_t channels_last, const aa_tensor_desc* out, int filter, int align, const OutEpi& epi, cudaStream_t stream,
+                 int32_t* launches) {
+  const int64_t es = dtype == AA_U8 ? 1 : 4;
+  const int Ci = channels_last ? (int)channels : 1;
+  const int64_t owf = out->w * Ci;
+  const int64_t tiles_x = (owf + TW - 1) / TW, tiles_y = (out->h + TH - 1) / TH;
+  if (tiles_x * tiles_y >= (1ll << 31)) return fail(AA_ERR_UNSUPPORTED, "aa_resize_crops: output too large for one launch");
+  std::unique_ptr<CropParams> hold(new CropParams);  // ~25 KB, kept off the stack; each launch copies it
+  CropParams& P = *hold;
+  P.out = out->data;
+  P.epi = epi;
+  P.out_sn = out->stride_n; P.out_sc = out->stride_c; P.out_sh = out->stride_h; P.out_sw = out->stride_w;
+  P.oH = (int)out->h; P.oW = (int)out->w; P.Ci = Ci; P.filter = filter; P.tiles_x = (int)tiles_x;
+  for (int32_t first = 0; first < count; first += kCropsPerLaunch) {
+    const int n = (int)std::min<int64_t>(kCropsPerLaunch, (int64_t)count - first);
+    P.first = first;
+    for (int k = 0; k < n; k++) {
+      const aa_image_desc& m = images[first + k];
+      const aa_crop& b = crops[first + k];
+      CropDesc& d = P.c[k];
+      d.src = (const char*)m.data + (b.top * m.stride_h + b.left * Ci) * es;
+      d.stride_h = m.stride_h;
+      d.stride_c = channels_last ? 0 : m.stride_c;
+      d.h = (int32_t)b.height; d.w = (int32_t)b.width;
+      d.scale_h = host_scale_f32(b.height, out->h, align);
+      d.scale_w = host_scale_f32(b.width, out->w, align);
+      d.kh = (int16_t)host_interp_size(b.height, out->h, filter, align, AA_F32);
+      d.kw = (int16_t)host_interp_size(b.width, out->w, filter, align, AA_F32);
+      d.hflip = b.hflip ? 1 : 0;
+    }
+    const dim3 grid((unsigned)(tiles_x * tiles_y), (unsigned)(channels_last ? 1 : channels), (unsigned)n);
+    if (dtype == AA_U8) aa_crops_kernel<uint8_t><<<grid, TW * NTY, 0, stream>>>(P);
+    else aa_crops_kernel<float><<<grid, TW * NTY, 0, stream>>>(P);
+    AA_LAUNCH_CHECK("aa_crops_kernel");
+    (*launches)++;
+  }
+  return AA_OK;
+}
+
+}  // namespace aa

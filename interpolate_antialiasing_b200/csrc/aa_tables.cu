@@ -15,16 +15,13 @@
 #include <tuple>
 
 #include "aa_common.cuh"
+#include "aa_window.cuh"
 
 namespace aa {
 
 // ------------------------------------------------------------------------------------------------
 // scalar recipe shared by host (launch planning) and device (the tables)
 // ------------------------------------------------------------------------------------------------
-__host__ __device__ inline double base_half(int filter) {  // interp_size * 0.5  (:208)
-  return filter == AA_FILTER_BOX ? 0.5 : (filter == AA_FILTER_TRIANGLE ? 1.0 : 2.0);
-}
-
 // host versions: plain IEEE float/double operators (no a*b+c pattern exists in them)
 // area_pixel_compute_scale<scalar_t> + compute_scales_value (ATen/native/UpSample.h): a caller-provided scale factor
 // (`scale_factors`, aa_interpolation_impl.h:735,740-742) replaces in/out by 1/scale_factor unless align_corners.
@@ -53,6 +50,8 @@ int host_interp_size(int64_t in, int64_t out, int filter, int align, int dtype, 
   float s = h_support_f32(h_scale_f32(in, out, align, user_scale), filter);
   return (int)ceilf(s) * 2 + 1;
 }
+
+float host_scale_f32(int64_t in, int64_t out, int align) { return h_scale_f32(in, out, align); }
 
 // Integer tables on the host: the same IEEE operations as the device kernels below (this TU is compiled with
 // -ffp-contract=off and x86-64 SSE arithmetic has no excess precision), so launch planning never has to read the
@@ -89,30 +88,6 @@ void host_int_tables(int64_t in, int64_t out, int filter, int align, int dtype, 
 // ------------------------------------------------------------------------------------------------
 // device filters, explicit rounding
 // ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ float filt_f32(int filter, float x) {
-  if (filter == AA_FILTER_BOX) return (x > -0.5f && x <= 0.5f) ? 1.0f : 0.0f;  // :367-372
-  if (x < 0.0f) x = -x;
-  if (filter == AA_FILTER_TRIANGLE) {  // :292-300, `1.0 - x` in double
-    return x < 1.0f ? __double2float_rn(__dsub_rn(1.0, (double)x)) : 0.0f;
-  }
-  if (x < 1.0f) {  // :417 all double: ((a+2)x - (a+3)) x x + 1, a = -0.5
-    double xd = (double)x;
-    double t = __dsub_rn(__dmul_rn(1.5, xd), 2.5);
-    t = __dmul_rn(t, xd);
-    t = __dmul_rn(t, xd);
-    return __double2float_rn(__dadd_rn(t, 1.0));
-  }
-  if (x < 2.0f) {  // :420 polynomial in float, final *a in double
-    float p = __fsub_rn(x, 5.0f);
-    p = __fmul_rn(p, x);
-    p = __fadd_rn(p, 8.0f);
-    p = __fmul_rn(p, x);
-    p = __fsub_rn(p, 4.0f);
-    return __double2float_rn(__dmul_rn((double)p, -0.5));
-  }
-  return 0.0f;
-}
-
 __device__ __forceinline__ double filt_f64(int filter, double x) {
   if (filter == AA_FILTER_BOX) return (x > -0.5 && x <= 0.5) ? 1.0 : 0.0;
   if (x < 0.0) x = -x;
@@ -134,38 +109,13 @@ __device__ __forceinline__ double filt_f64(int filter, double x) {
   return 0.0;
 }
 
-// One thread per output index.  fp32 instantiation of :194-281.
-// `scale` = area_pixel_compute_scale<float>, one IEEE division done by the host (h_scale_f32).
+// One thread per output index.  fp32 instantiation of :194-281 (aa_window.cuh).
 __global__ void aa_tables_fwd_f32(int64_t in, int64_t out, int filter, float scale, int K,
                                   int32_t* __restrict__ xmin_o, int32_t* __restrict__ xsize_o,
                                   float* __restrict__ w) {
   int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= out) return;
-  const double bh = base_half(filter);
-  const float support = (scale >= 1.0f) ? __double2float_rn(__dmul_rn(bh, (double)scale)) : (float)bh;  // :208-209
-  const float invscale = (scale >= 1.0f) ? __double2float_rn(__ddiv_rn(1.0, (double)scale)) : 1.0f;     // :242
-  const float center = __double2float_rn(__dmul_rn((double)scale, __dadd_rn((double)i, 0.5)));         // :253
-  long long xmin = __double2ll_rz(__dadd_rn((double)__fsub_rn(center, support), 0.5));                  // :254
-  if (xmin < 0) xmin = 0;
-  long long xmax = __double2ll_rz(__dadd_rn((double)__fadd_rn(center, support), 0.5));                  // :255-257
-  if (xmax > in) xmax = in;
-  xmax -= xmin;
-  xmin_o[i] = (int32_t)xmin;
-  xsize_o[i] = (int32_t)xmax;
-  float* wr = w + i * K;
-  float total = 0.0f;
-  long long j = 0;
-  for (; j < xmax && j < K; j++) {
-    float d = __fsub_rn(__ll2float_rn(j + xmin), center);                                               // :266
-    float arg = __double2float_rn(__dmul_rn(__dadd_rn((double)d, 0.5), (double)invscale));
-    float wj = filt_f32(filter, arg);
-    wr[j] = wj;
-    total = __fadd_rn(total, wj);                                                                      // :268
-  }
-  const long long nt = j;
-  if (total != 0.0f)
-    for (j = 0; j < nt; j++) wr[j] = __fdiv_rn(wr[j], total);                                           // :270-274
-  for (j = nt; j < K; j++) wr[j] = 0.0f;                                                                // :276-278
+  aa_window_f32(in, filter, scale, K, i, xmin_o + i, xsize_o + i, w + i * K);
 }
 
 __global__ void aa_tables_fwd_f64(int64_t in, int64_t out, int filter, double scale, int K,
