@@ -235,6 +235,33 @@ int aa_resize_crops(const aa_image_desc* images, const aa_crop* crops, int32_t c
                     int32_t channels_last, const aa_tensor_desc* out, int filter, int align_corners, uint32_t flags,
                     const aa_epilogue* epilogue, void* cuda_stream, int32_t* launches_out);
 
+/* Batched resize-then-crop: the evaluation transforms of an input pipeline, Resize(size) followed by CenterCrop, FiveCrop or
+ * TenCrop, with a resized size per crop and the crop taken after the resize (torchvision's crop(resize(img, ...), ...);
+ * not in the reference).  out[i] is the (oH, oW) window at (crop_top, crop_left) of
+ *     R_i = aa_resize_forward_ex(image_i[top:top+height, left:left+width] -> (resized_h, resized_w))
+ * bit for bit the AA_FLAG_FORCE_GENERAL arithmetic (table scales height/resized_h and width/resized_w, or the align_corners
+ * form; output index crop_top + oy of R_i has the window the table kernel builds for that index), flipped as `flip` says:
+ * bit 0 stores column ox at oW-1-ox, bit 1 stores row oy at oH-1-oy; channels keep their order.  That is
+ * hflip(crop(resize(img))), what TenCrop computes after Resize.  Only the window's outputs are computed.
+ *   - inputs, out dtypes and layouts, epilogue, flags, launches (ceil(count / 512)), graph capturability and the reads
+ *     staying inside the box are those of aa_resize_crops.  aa_resize_crops(c) is aa_resize_crops_ex with
+ *     resized = (oH, oW), crop_top = crop_left = 0 and flip = (hflip != 0), bit for bit;
+ *   - AA_ERR_INVALID (message names the crop index) for everything aa_resize_crops refuses with it, and for resized_h or
+ *     resized_w < 1, a window outside the resized image (crop_top < 0, crop_left < 0, crop_top + oH > resized_h,
+ *     crop_left + oW > resized_w: no zero padding) and flip bits other than 0 and 1; AA_ERR_UNSUPPORTED for everything
+ *     aa_resize_crops refuses with it (the 65-tap bound applies to box -> resized) and resized_h or resized_w >= 2^31.
+ *     Every check happens before the first launch;
+ *   - count == 0 is a no-op. */
+typedef struct aa_crop_ex {
+  int64_t top, left, height, width; /* box in the image that is resized (the whole image for Resize + CenterCrop)   */
+  int64_t resized_h, resized_w;     /* the size that box is resized to (torchvision Resize's output size)            */
+  int64_t crop_top, crop_left;      /* origin, in the resized image, of the (oH, oW) window stored in out[i]          */
+  int32_t flip;                     /* bit 0: flip the stored window horizontally, bit 1: vertically                  */
+} aa_crop_ex;
+int aa_resize_crops_ex(const aa_image_desc* images, const aa_crop_ex* crops, int32_t count, int32_t dtype, int64_t channels,
+                       int32_t channels_last, const aa_tensor_desc* out, int filter, int align_corners, uint32_t flags,
+                       const aa_epilogue* epilogue, void* cuda_stream, int32_t* launches_out);
+
 /* grad_in = Wh^T * grad_out * Ww : the true adjoint of aa_resize_forward, gather form, no atomics,
  * no zero-fill pass.  Replaces ti_upsample_bilinear2d_backward_cpu,
  * aa_interpolation_backward_impl.h:185-219 (linear_backward), whose body is the NON-antialiased

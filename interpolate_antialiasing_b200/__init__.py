@@ -12,13 +12,15 @@ calling needs the built extension and a CUDA device and fails loudly otherwise.
     aa_interp = aa.load()          # the pybind module itself, e.g. to pass to the reference's test.py helpers
 """
 import importlib.util
+import numbers
 import os
 
 from . import capi
 from ._build_ext import EXT, EXT_NAME, LIB
 
 __all__ = ["load", "linear_forward", "cubic_forward", "nearest_forward", "linear_backward", "cubic_backward",
-           "nearest_backward", "linear_backward_nonaa", "forward_with_flags", "resize_to_uint8", "decode_resize_normalize", "resized_crops", "AAResize", "aa_resize", "capi"]
+           "nearest_backward", "linear_backward_nonaa", "forward_with_flags", "resize_to_uint8", "decode_resize_normalize", "resized_crops", "resized_output_size",
+           "resize_center_crop", "five_crop", "ten_crop", "AAResize", "aa_resize", "capi"]
 
 _ext = None
 
@@ -101,6 +103,28 @@ def decode_resize_normalize(x_hwc_u8, output_size, mean, std, mode="bilinear", o
     return capi.resize_forward_ex(x, output_size, mode, out, scale, bias, align_corners)
 
 
+def _image_list(images):
+    """The `images` argument of resized_crops and the eval-crop helpers as a list of 3-D CUDA tensors."""
+    import torch
+    if torch.is_tensor(images):
+        assert images.dim() == 4 and images.is_cuda
+        cl = images.is_contiguous(memory_format=torch.channels_last) and not images.is_contiguous()
+        images = [t.permute(1, 2, 0) if cl else t for t in images.unbind(0)]
+    return images
+
+
+def _normalize_args(mean, std, out_dtype):
+    """-> (scale, bias, out dtype, flags) of the (x/255 - mean)/std epilogue, or none of it."""
+    import torch
+    scale = bias = None
+    if mean is not None or std is not None:
+        scale = [1.0 / (255.0 * s) for s in std]
+        bias = [-m / s for m, s in zip(mean, std)]
+        out_dtype = out_dtype or torch.float16
+    out_dtype = out_dtype or torch.float32
+    return scale, bias, out_dtype, capi.FLAG_ROUND_NEAREST if out_dtype == torch.uint8 else capi.FLAG_AUTO
+
+
 def resized_crops(images, boxes, size, mode="bilinear", hflip=None, mean=None, std=None, out_dtype=None, align_corners=False):
     """RandomResizedCrop + RandomHorizontalFlip of a batch in one kernel launch: torchvision's
     `resized_crop(img, top, left, height, width, size, antialias=True)` per image, with its own box, optionally flipped.
@@ -115,10 +139,7 @@ def resized_crops(images, boxes, size, mode="bilinear", hflip=None, mean=None, s
             out_dtype=torch.uint8.
     Returns a contiguous [N,C,oH,oW] tensor."""
     import torch
-    if torch.is_tensor(images):
-        assert images.dim() == 4 and images.is_cuda
-        cl = images.is_contiguous(memory_format=torch.channels_last) and not images.is_contiguous()
-        images = [t.permute(1, 2, 0) if cl else t for t in images.unbind(0)]
+    images = _image_list(images)
     if isinstance(boxes, torch.Tensor):
         boxes = boxes.tolist()
     if hflip is not None and isinstance(hflip, torch.Tensor):
@@ -126,15 +147,134 @@ def resized_crops(images, boxes, size, mode="bilinear", hflip=None, mean=None, s
     oH, oW = (int(size), int(size)) if isinstance(size, int) else (int(size[0]), int(size[1]))
     hwc = capi._is_hwc(images[0])
     C = images[0].shape[-1] if hwc else images[0].shape[0]
-    scale = bias = None
-    if mean is not None or std is not None:
-        scale = [1.0 / (255.0 * s) for s in std]
-        bias = [-m / s for m, s in zip(mean, std)]
-        out_dtype = out_dtype or torch.float16
-    out = torch.empty((len(images), C, oH, oW), dtype=out_dtype or torch.float32, device=images[0].device)
-    flags = capi.FLAG_ROUND_NEAREST if out.dtype == torch.uint8 else capi.FLAG_AUTO
+    scale, bias, out_dtype, flags = _normalize_args(mean, std, out_dtype)
+    out = torch.empty((len(images), C, oH, oW), dtype=out_dtype, device=images[0].device)
     return capi.resize_crops(images, boxes, (oH, oW), mode, out=out, hflip=hflip, scale=scale, bias=bias,
                              align_corners=align_corners, flags=flags)[0]
+
+
+def resized_output_size(h, w, size, max_size=None):
+    """The (height, width) torchvision.transforms.v2.functional.resize(img, size, max_size=max_size) gives an h x w image,
+    host-only.  size: an int or [int] for the shorter edge (the longer one becomes int(size * long / short), the aspect ratio
+    kept), (h, w) for both, or None with max_size (the longer edge becomes max_size).  max_size caps the longer edge of the
+    int / [int] form and must then exceed the requested shorter edge; it cannot be combined with (h, w)."""
+    if isinstance(size, numbers.Integral):
+        size = [int(size)]
+    elif size is not None:
+        size = [int(v) for v in size]
+        if len(size) not in (1, 2):
+            raise ValueError(f"size must be an int or a sequence of one or two ints, got {size}")
+        if max_size is not None and len(size) != 1:
+            raise ValueError("max_size should only be passed if size is None or specifies the length of the smaller edge, "
+                             "i.e. size should be an int or a sequence of length 1")
+    short, long = (w, h) if w <= h else (h, w)
+    if size is None:
+        if not isinstance(max_size, numbers.Integral):
+            raise ValueError(f"max_size must be an integer when size is None, but got {max_size} instead.")
+        new_short, new_long = int(max_size * short / long), int(max_size)
+    elif len(size) == 1:
+        new_short, new_long = size[0], int(size[0] * long / short)
+        if max_size is not None:
+            if max_size <= size[0]:
+                raise ValueError(f"max_size = {max_size} must be strictly greater than the requested size for the smaller "
+                                 f"edge size = {size}")
+            if new_long > max_size:
+                new_short, new_long = int(max_size * new_short / new_long), int(max_size)
+    else:
+        return size[0], size[1]
+    return (new_long, new_short) if w <= h else (new_short, new_long)
+
+
+def _crop_hw(crop_size):
+    """torchvision's CenterCrop / FiveCrop size argument: an int, [int] or (h, w)."""
+    if isinstance(crop_size, numbers.Integral):
+        return int(crop_size), int(crop_size)
+    crop_size = [int(v) for v in crop_size]
+    if len(crop_size) == 1:
+        return crop_size[0], crop_size[0]
+    if len(crop_size) != 2:
+        raise ValueError(f"crop size must be an int or (h, w), got {crop_size}")
+    return crop_size[0], crop_size[1]
+
+
+def _eval_crops(hw, size, crop_size, kind, vertical_flip=False, max_size=None):
+    """Host-only: the aa_crop_ex rows ([N, kinds] of capi.crop_ex_dtype) of Resize(size, max_size) followed by
+    CenterCrop ("center"), FiveCrop ("five") or TenCrop ("ten") of crop_size, for images of sizes hw ([N, 2]: h, w)."""
+    import numpy as np
+    ch, cw = _crop_hw(crop_size)
+    hw = np.asarray(hw, np.int64).reshape(-1, 2)
+    R = np.array([resized_output_size(int(h), int(w), size, max_size) for h, w in hw], np.int64).reshape(-1, 2)
+    small = np.nonzero((R[:, 0] < ch) | (R[:, 1] < cw))[0]
+    if len(small):
+        i = int(small[0])
+        raise ValueError(f"crop size {(ch, cw)} is larger than the resized image {tuple(int(v) for v in R[i])} of image {i}: "
+                         "zero padding is not supported")
+    dy, dx = R[:, 0] - ch, R[:, 1] - cw
+    # torchvision's anchor int(round(d / 2.0)): Python's round, half to even, which np.round also does
+    cy, cx = np.round(dy / 2.0).astype(np.int64), np.round(dx / 2.0).astype(np.int64)
+    z = np.zeros_like(dy)
+    five = [(z, z, 0), (z, dx, 0), (dy, z, 0), (dy, dx, 0), (cy, cx, 0)]  # torchvision's order: tl, tr, bl, br, center
+    if kind == "center":
+        windows = five[4:]
+    elif kind == "five":
+        windows = five
+    elif kind == "ten":
+        # a crop of the flipped resized image is the flip of the mirrored window of the unflipped one
+        windows = five + [(dy - t, l, 2) if vertical_flip else (t, dx - l, 1) for t, l, _ in five]
+    else:
+        raise ValueError(f"unknown crop kind {kind!r}")
+    crops = np.zeros((len(hw), len(windows)), capi.crop_ex_dtype())
+    crops["height"], crops["width"] = hw[:, :1], hw[:, 1:]
+    crops["resized_h"], crops["resized_w"] = R[:, :1], R[:, 1:]
+    for j, (top, left, flip) in enumerate(windows):
+        crops["crop_top"][:, j], crops["crop_left"][:, j], crops["flip"][:, j] = top, left, flip
+    return crops
+
+
+def _resize_then_crop(images, size, crop_size, kind, vertical_flip, mode, max_size, mean, std, out_dtype):
+    """_eval_crops of every image in one aa_resize_crops_ex call (ceil(crops / 512) launches) -> [N * kinds, C, ch, cw]."""
+    import numpy as np
+    import torch
+    images = _image_list(images)
+    hwc = capi._is_hwc(images[0])
+    C = images[0].shape[-1] if hwc else images[0].shape[0]
+    hw = [(t.shape[0], t.shape[1]) if hwc else (t.shape[1], t.shape[2]) for t in images]
+    crops = _eval_crops(hw, size, crop_size, kind, vertical_flip, max_size)
+    scale, bias, out_dtype, flags = _normalize_args(mean, std, out_dtype)
+    ch, cw = _crop_hw(crop_size)
+    out = torch.empty((crops.size, C, ch, cw), dtype=out_dtype, device=images[0].device)
+    rows = np.repeat(capi.image_descs(images, hwc), crops.shape[1])
+    capi.launch_crops_ex(rows, crops.reshape(-1), capi._dtype_code(images[0]), C, hwc, out, mode, scale, bias, flags=flags)
+    return out
+
+
+def resize_center_crop(images, size, crop_size, mode="bilinear", max_size=None, mean=None, std=None, out_dtype=None):
+    """The evaluation transform CenterCrop(crop_size)(Resize(size, antialias=True, max_size=max_size)(img)) of a batch in
+    one kernel launch: every image resized with its own aspect ratio (resized_output_size), then the centre window at
+    torchvision's anchor int(round((R - c) / 2.0)) stored; only the window's outputs are computed.  images, mode, mean/std
+    and out_dtype as in resized_crops.  A crop larger than a resized image raises ValueError (torchvision would zero-pad).
+    Returns a contiguous [N,C,ch,cw] tensor."""
+    return _resize_then_crop(images, size, crop_size, "center", False, mode, max_size, mean, std, out_dtype)
+
+
+def five_crop(images, size, crop_size, mode="bilinear", max_size=None, mean=None, std=None, out_dtype=None):
+    """FiveCrop(crop_size) after Resize(size, antialias=True, max_size=max_size), one kernel launch per 512 crops.
+    Returns a contiguous [N,5,C,ch,cw] tensor in torchvision's order: top-left, top-right, bottom-left, bottom-right,
+    centre.  Other arguments as in resize_center_crop."""
+    y = _resize_then_crop(images, size, crop_size, "five", False, mode, max_size, mean, std, out_dtype)
+    return y.view(-1, 5, *y.shape[1:])
+
+
+def ten_crop(images, size, crop_size, vertical_flip=False, mode="bilinear", max_size=None, mean=None, std=None,
+             out_dtype=None):
+    """TenCrop(crop_size, vertical_flip) after Resize(size, antialias=True, max_size=max_size), one kernel launch per 512
+    crops.  Returns a contiguous [N,10,C,ch,cw] tensor in torchvision's order: the five crops of five_crop, then the five
+    crops of the flipped resized image.  Each of those is computed as the flip of the mirrored window of the unflipped
+    image: the flipped top-left is the flipped window at left = W - cw, the flipped centre the one at
+    left = W - cw - round((W - cw) / 2), one column right of the unflipped centre when W - cw is odd (rows and the
+    vertical flip likewise).  Other arguments as in resize_center_crop."""
+    y = _resize_then_crop(images, size, crop_size, "ten", vertical_flip, mode, max_size, mean, std, out_dtype)
+    return y.view(-1, 10, *y.shape[1:])
 
 
 from .functional import AAResize, aa_resize  # noqa: E402

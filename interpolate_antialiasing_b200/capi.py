@@ -19,7 +19,7 @@ FILTERS = {"nearest": BOX, "box": BOX, "bilinear": TRIANGLE, "linear": TRIANGLE,
 
 EXPORTS = [
     "aa_abi_version", "aa_last_error", "aa_interp_size", "aa_host_tables", "aa_build_tables", "aa_build_tables_sf", "aa_warm_tables",
-    "aa_clear_table_cache", "aa_check_device", "aa_debug_counters", "aa_resize_forward", "aa_resize_forward_sf", "aa_resize_backward_sf", "aa_resize_forward_ex", "aa_resize_forward_ragged", "aa_resize_crops", "aa_resize_backward",
+    "aa_clear_table_cache", "aa_check_device", "aa_debug_counters", "aa_resize_forward", "aa_resize_forward_sf", "aa_resize_backward_sf", "aa_resize_forward_ex", "aa_resize_forward_ragged", "aa_resize_crops", "aa_resize_crops_ex", "aa_resize_backward",
     "aa_resize_backward_nonaa_bilinear", "aa_resize_forward_host", "aa_resize_forward_host_multi", "aa_launch_count",
 ]
 
@@ -49,6 +49,28 @@ class Crop(ctypes.Structure):
     """aa_crop: a box (top, left, height, width) in pixels of its image and an optional horizontal flip."""
     _fields_ = [("top", ctypes.c_int64), ("left", ctypes.c_int64), ("height", ctypes.c_int64), ("width", ctypes.c_int64),
                 ("hflip", ctypes.c_int32)]
+
+
+class CropEx(ctypes.Structure):
+    """aa_crop_ex: a box of its image, the size it is resized to, the origin of the stored window in the resized image and
+    the flip bits (0: horizontal, 1: vertical)."""
+    _fields_ = [("top", ctypes.c_int64), ("left", ctypes.c_int64), ("height", ctypes.c_int64), ("width", ctypes.c_int64),
+                ("resized_h", ctypes.c_int64), ("resized_w", ctypes.c_int64), ("crop_top", ctypes.c_int64),
+                ("crop_left", ctypes.c_int64), ("flip", ctypes.c_int32)]
+
+
+def crop_ex_dtype():
+    """numpy structured dtype laid out as aa_crop_ex (72 bytes): an array of it is passed to the C ABI as it stands, so a
+    batch of thousands of crops needs no ctypes object per crop."""
+    import numpy as np
+    return np.dtype([(f, np.int64) for f, _ in CropEx._fields_[:-1]] + [("flip", np.int32)], align=True)
+
+
+def image_desc_dtype():
+    """numpy structured dtype laid out as aa_image_desc (40 bytes)."""
+    import numpy as np
+    return np.dtype([("data", np.uint64), ("h", np.int64), ("w", np.int64), ("stride_h", np.int64), ("stride_c", np.int64)],
+                    align=True)
 
 
 class Scales(ctypes.Structure):
@@ -85,6 +107,7 @@ def lib():
         L.aa_resize_forward_ex.argtypes = [P(TensorDesc), P(TensorDesc), i32, i32, u32, P(Epilogue), vp]
         L.aa_resize_forward_ragged.argtypes = [P(ImageDesc), i32, i32, i64, i32, P(TensorDesc), i32, i32, u32, P(Epilogue), vp, P(i32)]
         L.aa_resize_crops.argtypes = [P(ImageDesc), P(Crop), i32, i32, i64, i32, P(TensorDesc), i32, i32, u32, P(Epilogue), vp, P(i32)]
+        L.aa_resize_crops_ex.argtypes = [vp, vp, i32, i32, i64, i32, P(TensorDesc), i32, i32, u32, P(Epilogue), vp, P(i32)]
         L.aa_resize_backward.argtypes = [P(TensorDesc), P(TensorDesc), i32, i32, u32, vp]
         L.aa_resize_backward_nonaa_bilinear.argtypes = [P(TensorDesc), P(TensorDesc), i32, vp]
         L.aa_resize_forward_host.argtypes = [P(TensorDesc), P(TensorDesc), i32, i32, u32]
@@ -284,6 +307,70 @@ def resize_crops(images, boxes, output_size, filter, out=None, hflip=None, scale
     check(lib().aa_resize_crops(arr, crops, n, dtype, C, int(hwc), ctypes.byref(do), _filter(filter), int(align_corners), flags,
                                 ctypes.byref(e), _stream(out), ctypes.byref(k)))
     return out, k.value
+
+
+def image_descs(images, hwc):
+    """aa_image_desc rows (an image_desc_dtype array) of a list of [H,W,C] (hwc) or [C,H,W] CUDA tensors."""
+    import numpy as np
+    if hwc:
+        rows = [(t.data_ptr(), t.shape[0], t.shape[1], t.stride(0), 1) for t in images]
+    else:
+        rows = [(t.data_ptr(), t.shape[1], t.shape[2], t.stride(1), t.stride(0)) for t in images]
+    return np.array(rows, dtype=image_desc_dtype())
+
+
+def crop_ex_array(crops):
+    """aa_crop_ex rows (a crop_ex_dtype array) from (top, left, height, width, resized_h, resized_w, crop_top, crop_left, flip)
+    tuples, an [N, 9] integer array or a crop_ex_dtype array."""
+    import numpy as np
+    if isinstance(crops, np.ndarray) and crops.dtype == crop_ex_dtype():
+        return np.ascontiguousarray(crops.reshape(-1))
+    rows = np.asarray(crops, dtype=np.int64).reshape(-1, 9)
+    arr = np.zeros(rows.shape[0], crop_ex_dtype())
+    for k, f in enumerate(arr.dtype.names):
+        arr[f] = rows[:, k]
+    if not np.array_equal(arr["flip"], rows[:, 8]):
+        raise ValueError("crop_ex_array: flip does not fit in 32 bits")
+    return arr
+
+
+def launch_crops_ex(image_rows, crop_rows, dtype, channels, hwc, out, filter, scale=None, bias=None, align_corners=False,
+                    flags=FLAG_AUTO):
+    """aa_resize_crops_ex on descriptor arrays (image_descs / crop_ex_array, one row per crop) into `out`; -> launches."""
+    assert len(image_rows) == len(crop_rows) and image_rows.dtype == image_desc_dtype() and crop_rows.dtype == crop_ex_dtype()
+    assert image_rows.flags.c_contiguous and crop_rows.flags.c_contiguous
+    e = _epilogue(scale, bias)
+    k = ctypes.c_int32(0)
+    do = desc(out)
+    check(lib().aa_resize_crops_ex(image_rows.ctypes.data, crop_rows.ctypes.data, len(crop_rows), dtype, channels, int(hwc),
+                                   ctypes.byref(do), _filter(filter), int(align_corners), flags, ctypes.byref(e), _stream(out),
+                                   ctypes.byref(k)))
+    return k.value
+
+
+def resize_crops_ex(images, crops, output_size, filter, out=None, scale=None, bias=None, align_corners=False, flags=FLAG_AUTO):
+    """Batched resize-then-crop (aa_resize_crops_ex): out[i] = the output_size window at (crop_top, crop_left) of
+    resize(images[i][top:top+height, left:left+width]) to (resized_h, resized_w), flipped horizontally where bit 0 of flip is
+    set and vertically where bit 1 is.  `images` as in resize_crops; `crops`: one aa_crop_ex row per image, tuples
+    (top, left, height, width, resized_h, resized_w, crop_top, crop_left, flip), an [N, 9] integer array or a crop_ex_dtype
+    array.  `out` defaults to a contiguous float32 [N,C,oH,oW]; scale/bias as in resize_crops.  Returns (out, launches)."""
+    import torch
+    n = len(images)
+    rows = crop_ex_array(crops)
+    if len(rows) != n:
+        raise ValueError("resize_crops_ex: images and crops must have the same length")
+    hwc = bool(n) and _is_hwc(images[0])
+    if n:
+        C = images[0].shape[-1] if hwc else images[0].shape[0]
+    elif out is not None:
+        C = out.shape[1]
+    else:
+        raise ValueError("resize_crops_ex: an empty batch needs `out`")
+    oH, oW = int(output_size[0]), int(output_size[1])
+    if out is None:
+        out = torch.empty((n, C, oH, oW), dtype=torch.float32, device=images[0].device)
+    dtype = _dtype_code(images[0]) if n else F32
+    return out, launch_crops_ex(image_descs(images, hwc), rows, dtype, C, hwc, out, filter, scale, bias, align_corners, flags)
 
 
 def resize_backward(grad_out, input_size, filter, align_corners=False, nonaa=False, flags=FLAG_AUTO, scales=None, out=None):

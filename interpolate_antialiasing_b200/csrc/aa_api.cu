@@ -451,23 +451,29 @@ int aa_resize_forward_ragged(const aa_image_desc* images, int32_t count, int32_t
   return AA_OK;
 }
 
-int aa_resize_crops(const aa_image_desc* images, const aa_crop* crops, int32_t count, int32_t dtype, int64_t channels,
-                    int32_t channels_last, const aa_tensor_desc* out, int filter, int align_corners, uint32_t flags,
-                    const aa_epilogue* epilogue, void* cuda_stream, int32_t* launches_out) {
+static_assert(sizeof(aa_crop_ex) == 72, "aa_crop_ex layout (capi.CropEx and capi.crop_ex_dtype() mirror it)");
+
+// aa_resize_crops and aa_resize_crops_ex: every check before the first launch, then the crops kernel.  `name` prefixes
+// the messages.
+static int resize_crops_impl(const char* name, const aa_image_desc* images, const aa_crop_ex* crops, int32_t count,
+                             int32_t dtype, int64_t channels, int32_t channels_last, const aa_tensor_desc* out, int filter,
+                             int align_corners, uint32_t flags, const aa_epilogue* epilogue, void* cuda_stream,
+                             int32_t* launches_out) {
   int rc;
+  const std::string nm = name;
   if (launches_out) *launches_out = 0;
-  if (count < 0 || (count > 0 && (!images || !crops))) return fail(AA_ERR_INVALID, "aa_resize_crops: null image or crop list");
+  if (count < 0 || (count > 0 && (!images || !crops))) return fail(AA_ERR_INVALID, nm + ": null image or crop list");
   if ((rc = check_desc(out, "output")) != AA_OK) return rc;
   if ((rc = check_filter(filter)) != AA_OK) return rc;
-  if (dtype == AA_F64) return fail(AA_ERR_UNSUPPORTED, "aa_resize_crops: input dtype must be u8 or f32");
-  if (dtype != AA_U8 && dtype != AA_F32) return fail(AA_ERR_INVALID, "aa_resize_crops: input dtype must be u8 or f32");
+  if (dtype == AA_F64) return fail(AA_ERR_UNSUPPORTED, nm + ": input dtype must be u8 or f32");
+  if (dtype != AA_U8 && dtype != AA_F32) return fail(AA_ERR_INVALID, nm + ": input dtype must be u8 or f32");
   if (flags & (AA_FLAG_FORCE_STREAM | AA_FLAG_STREAM_TMA | AA_FLAG_STREAM_LDG | AA_FLAG_VMMA | AA_FLAG_FORCE_GENERAL))
-    return fail(AA_ERR_UNSUPPORTED, "aa_resize_crops: has one kernel; the path-forcing flags do not apply");
+    return fail(AA_ERR_UNSUPPORTED, nm + ": has one kernel; the path-forcing flags do not apply");
   if (channels < 1 || out->n != count || out->c != channels)
-    return fail(AA_ERR_INVALID, "aa_resize_crops: output must be [count, channels, oH, oW]");
+    return fail(AA_ERR_INVALID, nm + ": output must be [count, channels, oH, oW]");
   const int64_t ci = channels_last ? channels : 1;
-  if (out->h >= (1ll << 31) || out->w * ci >= (1ll << 31)) return fail(AA_ERR_UNSUPPORTED, "aa_resize_crops: output plane too large");
-  if (!channels_last && channels > 65535) return fail(AA_ERR_UNSUPPORTED, "aa_resize_crops: more than 65535 planar channels");
+  if (out->h >= (1ll << 31) || out->w * ci >= (1ll << 31)) return fail(AA_ERR_UNSUPPORTED, nm + ": output plane too large");
+  if (!channels_last && channels > 65535) return fail(AA_ERR_UNSUPPORTED, nm + ": more than 65535 planar channels");
   OutEpi epi;
   epi.round = (flags & AA_FLAG_ROUND_NEAREST) ? 1 : 0;
   switch (out->dtype) {
@@ -475,7 +481,7 @@ int aa_resize_crops(const aa_image_desc* images, const aa_crop* crops, int32_t c
     case AA_U8: epi.kind = 1; break;
     case AA_F16: epi.kind = 2; break;
     case AA_BF16: epi.kind = 3; break;
-    default: return fail(AA_ERR_INVALID, "aa_resize_crops: output dtype must be f32, u8, f16 or bf16");
+    default: return fail(AA_ERR_INVALID, nm + ": output dtype must be f32, u8, f16 or bf16");
   }
   if (epilogue && epilogue->normalize) {
     if (channels > 4) return fail(AA_ERR_UNSUPPORTED, "normalisation epilogue: at most 4 channels");
@@ -487,30 +493,59 @@ int aa_resize_crops(const aa_image_desc* images, const aa_crop* crops, int32_t c
   bool out_cl = false;
   if ((rc = classify_layout(*out, channels_last != 0, &lout, &out_cl)) != AA_OK) return rc;
   if (out_cl && !channels_last && channels > 1)
-    return fail(AA_ERR_UNSUPPORTED, "aa_resize_crops: a planar input needs a channels_first output");
+    return fail(AA_ERR_UNSUPPORTED, nm + ": a planar input needs a channels_first output");
   for (int32_t i = 0; i < count; i++) {
     const aa_image_desc& m = images[i];
-    const aa_crop& b = crops[i];
-    const std::string at = "aa_resize_crops: crop " + std::to_string(i);
+    const aa_crop_ex& b = crops[i];
+    const std::string at = nm + ": crop " + std::to_string(i);
     if (!m.data || m.h <= 0 || m.w <= 0) return fail(AA_ERR_INVALID, at + ": image is empty");
     if (m.stride_h < m.w * ci) return fail(AA_ERR_INVALID, at + ": rows of the image overlap");
     if (b.top < 0 || b.left < 0 || b.height < 1 || b.width < 1 || b.height > m.h - b.top || b.width > m.w - b.left)
       return fail(AA_ERR_INVALID, at + ": box (top " + std::to_string(b.top) + ", left " + std::to_string(b.left) + ", height " +
                                       std::to_string(b.height) + ", width " + std::to_string(b.width) + ") is not inside its " +
                                       std::to_string(m.h) + "x" + std::to_string(m.w) + " image");
+    if (b.resized_h < 1 || b.resized_w < 1)
+      return fail(AA_ERR_INVALID, at + ": resized size " + std::to_string(b.resized_h) + "x" + std::to_string(b.resized_w) +
+                                      " is empty");
+    if (b.crop_top < 0 || b.crop_left < 0 || b.crop_top > b.resized_h - out->h || b.crop_left > b.resized_w - out->w)
+      return fail(AA_ERR_INVALID, at + ": window (top " + std::to_string(b.crop_top) + ", left " + std::to_string(b.crop_left) +
+                                      ", " + std::to_string(out->h) + "x" + std::to_string(out->w) + ") is not inside the " +
+                                      std::to_string(b.resized_h) + "x" + std::to_string(b.resized_w) + " resized image");
+    if (b.flip & ~3) return fail(AA_ERR_INVALID, at + ": flip has bits other than 0 (horizontal) and 1 (vertical)");
     if (b.height >= (1ll << 31) || b.width >= (1ll << 31)) return fail(AA_ERR_UNSUPPORTED, at + ": box too large");
-    if (host_interp_size(b.height, out->h, filter, align_corners, AA_F32) > kCropMaxTaps ||
-        host_interp_size(b.width, out->w, filter, align_corners, AA_F32) > kCropMaxTaps)
+    if (b.resized_h >= (1ll << 31) || b.resized_w >= (1ll << 31)) return fail(AA_ERR_UNSUPPORTED, at + ": resized size too large");
+    if (host_interp_size(b.height, b.resized_h, filter, align_corners, AA_F32) > kCropMaxTaps ||
+        host_interp_size(b.width, b.resized_w, filter, align_corners, AA_F32) > kCropMaxTaps)
       return fail(AA_ERR_UNSUPPORTED, at + ": window longer than " + std::to_string(kCropMaxTaps) + " taps (downscale too large)");
   }
   if (count == 0) return AA_OK;
   DeviceGuard g(out->device);
   if (!g.ok) return cuda_fail(g.err, "cudaSetDevice");
   int32_t launches = 0;
-  rc = launch_crops(images, crops, count, dtype, channels, channels_last, out, filter, align_corners ? 1 : 0, epi,
+  rc = launch_crops(name, images, crops, count, dtype, channels, channels_last, out, filter, align_corners ? 1 : 0, epi,
                     (cudaStream_t)cuda_stream, &launches);
   if (launches_out) *launches_out = launches;
   return rc;
+}
+
+int aa_resize_crops_ex(const aa_image_desc* images, const aa_crop_ex* crops, int32_t count, int32_t dtype, int64_t channels,
+                       int32_t channels_last, const aa_tensor_desc* out, int filter, int align_corners, uint32_t flags,
+                       const aa_epilogue* epilogue, void* cuda_stream, int32_t* launches_out) {
+  return resize_crops_impl("aa_resize_crops_ex", images, crops, count, dtype, channels, channels_last, out, filter,
+                           align_corners, flags, epilogue, cuda_stream, launches_out);
+}
+
+int aa_resize_crops(const aa_image_desc* images, const aa_crop* crops, int32_t count, int32_t dtype, int64_t channels,
+                    int32_t channels_last, const aa_tensor_desc* out, int filter, int align_corners, uint32_t flags,
+                    const aa_epilogue* epilogue, void* cuda_stream, int32_t* launches_out) {
+  // each box resized to the output size, the window at the origin
+  std::vector<aa_crop_ex> ex(crops && count > 0 ? (size_t)count : 0);
+  for (size_t i = 0; i < ex.size(); i++) {
+    const aa_crop& b = crops[i];
+    ex[i] = aa_crop_ex{b.top, b.left, b.height, b.width, out ? out->h : 0, out ? out->w : 0, 0, 0, b.hflip ? 1 : 0};
+  }
+  return resize_crops_impl("aa_resize_crops", images, crops ? ex.data() : nullptr, count, dtype, channels, channels_last, out,
+                           filter, align_corners, flags, epilogue, cuda_stream, launches_out);
 }
 
 static int backward_impl(const aa_tensor_desc* gout, const aa_tensor_desc* gin, int filter, int align_corners, uint32_t flags,

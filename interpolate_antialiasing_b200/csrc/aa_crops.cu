@@ -1,6 +1,11 @@
-// aa_crops.cu -- batched resized crops (aa_resize_crops): one box per crop, any box size, one output size, one launch.
+// aa_crops.cu -- batched resized crops (aa_resize_crops, aa_resize_crops_ex): one box per crop, any box size, resized to
+// its own size, one (oH, oW) window of that resized image stored per crop, one launch.
 //
-//   out[n, c, oy, ox'] = sum_y sum_x Wh_n[oy, y] * Ww_n[ox, x] * image_n[top_n + y, left_n + x, c],  ox' = hflip ? oW-1-ox : ox
+//   out[n, c, oy', ox'] = sum_y sum_x Wh_n[y0_n + oy, y] * Ww_n[x0_n + ox, x] * image_n[top_n + y, left_n + x, c]
+//   oy' = vflip ? oH-1-oy : oy,  ox' = hflip ? oW-1-ox : ox
+//
+// Wh_n, Ww_n: the tables of box -> resized size; (y0_n, x0_n): the window origin in the resized image.  aa_resize_crops is
+// the case resized = (oH, oW), origin 0, no vertical flip.
 //
 // Random boxes almost never share a size, so table caches and per-size launch plans do not pay here: every CTA computes
 // the tables of its own tile (xmin, xsize and weights of its output rows and of its tile's pixel columns) into shared
@@ -9,8 +14,9 @@
 //
 // Arithmetic: the EXACT order of aa_general_kernel -- horizontal pass into shared T rounded to fp32, then the vertical
 // pass with ascending taps, separate multiply and add -- so every output is bit-identical to aa_resize_forward_ex on the
-// crop's view with AA_FLAG_FORCE_GENERAL.  Only the in-window taps inside the box are read, so NaN/Inf land exactly where
-// the reference puts them without the drain kernel behind the fast float paths.
+// crop's view with AA_FLAG_FORCE_GENERAL (to the resized size, then sliced to the window).  Only the in-window taps inside
+// the box are read, so NaN/Inf land exactly where the reference puts them without the drain kernel behind the fast float
+// paths.
 #include <algorithm>
 
 #include "aa_common.cuh"
@@ -27,16 +33,17 @@ constexpr int RC = 32;           // input rows per chunk
 constexpr int HPT = RC / NTY;    // horizontal-pass rows per thread per chunk
 constexpr int KP = kCropMaxTaps; // weight row pitch in shared memory (odd: the columns of a warp hit distinct banks)
 
-// One crop, 48 bytes.  src already points at the box's first element (top, left) of channel 0, offset in 64 bits.
+// One crop, 56 bytes.  src already points at the box's first element (top, left) of channel 0, offset in 64 bits.
 struct CropDesc {
   const void* src;
   int64_t stride_h, stride_c;  // elements; stride_c: between channel planes (planar input)
   int32_t h, w;                // box size
-  float scale_h, scale_w;      // fp32 table scales of the two axes (h_scale_f32 of box -> output)
+  int32_t y0, x0;              // origin of the stored window in the resized image
+  float scale_h, scale_w;      // fp32 table scales of the two axes (h_scale_f32 of box -> resized size)
   int16_t kh, kw;              // interp_size of the two axes (<= kCropMaxTaps)
-  int32_t hflip;
+  int32_t flip;                // bit 0: horizontal, bit 1: vertical
 };
-static_assert(sizeof(CropDesc) == 48, "CropDesc layout");
+static_assert(sizeof(CropDesc) == 56, "CropDesc layout");
 
 struct CropParams {
   void* out;
@@ -46,15 +53,17 @@ struct CropParams {
   int oH, oW, Ci, filter, tiles_x;
   CropDesc c[kCropsPerLaunch];
 };
-// sm_100 takes up to 32764 bytes of kernel parameters
+// sm_100 takes up to 32764 bytes of kernel parameters (512 x 56 bytes of descriptors + the header)
 static_assert(sizeof(CropParams) <= 32764, "kCropsPerLaunch too large for the kernel parameter space");
 
 template <typename in_t>
 __device__ __forceinline__ float ld_in(const in_t* p) { return (float)__ldg(p); }
 
 // One CTA: a TH x TW tile of the flat output (pixel columns x interleaved channels) of one plane of one crop.
+// 4 CTAs per SM (64 registers, 4 x 34 KB of shared memory): with no minimum given, ptxas still allocates 64 registers for
+// the uint8 instantiation but spills; with the minimum it fits them without spilling.
 template <typename in_t>
-__global__ void __launch_bounds__(TW* NTY) aa_crops_kernel(const __grid_constant__ CropParams P) {
+__global__ void __launch_bounds__(TW* NTY, 4) aa_crops_kernel(const __grid_constant__ CropParams P) {
   __shared__ float Ts[RC][TW + 1];
   __shared__ float sWh[TH][KP];
   __shared__ float sWw[TW][KP];
@@ -70,13 +79,13 @@ __global__ void __launch_bounds__(TW* NTY) aa_crops_kernel(const __grid_constant
   const int px0 = of0 / Ci;
   const int npx = (min(of0 + TW, owf) - 1) / Ci - px0 + 1;
 
-  // ---- the tile's tables, K1 arithmetic
+  // ---- the tile's tables, K1 arithmetic, at the tile's indices in the resized image
   for (int k = tid; k < TH + TW; k += TW * NTY) {
     if (k < TH) {
-      if (k < nrows) aa_window_f32(D.h, P.filter, D.scale_h, D.kh, oy0 + k, &sHs[k], &sHn[k], sWh[k]);
+      if (k < nrows) aa_window_f32(D.h, P.filter, D.scale_h, D.kh, D.y0 + oy0 + k, &sHs[k], &sHn[k], sWh[k]);
     } else if (k - TH < npx) {
       const int j = k - TH;
-      aa_window_f32(D.w, P.filter, D.scale_w, D.kw, px0 + j, &sWs[j], &sWn[j], sWw[j]);
+      aa_window_f32(D.w, P.filter, D.scale_w, D.kw, D.x0 + px0 + j, &sWs[j], &sWn[j], sWw[j]);
     }
   }
   __syncthreads();
@@ -136,27 +145,30 @@ __global__ void __launch_bounds__(TW* NTY) aa_crops_kernel(const __grid_constant
   }
   if (col_ok) {
     const int ch = plane + c;  // one of the two is 0
-    const int oxs = D.hflip ? P.oW - 1 - px : px;
-    const int64_t base = (P.first + blockIdx.z) * P.out_sn + ch * P.out_sc + oxs * P.out_sw;
+    const int oxs = (D.flip & 1) ? P.oW - 1 - px : px;
+    const bool vflip = D.flip & 2;
+    const int64_t sh = vflip ? -P.out_sh : P.out_sh;
+    const int64_t base = (P.first + blockIdx.z) * P.out_sn + ch * P.out_sc + oxs * P.out_sw +
+                         (int64_t)(vflip ? P.oH - 1 - oy0 : oy0) * P.out_sh;
 #pragma unroll
     for (int r = 0; r < RPT; r++) {
       const int oyl = ty + r * NTY;
-      if (oyl < nrows) aa_store<true>(P.out, base + (int64_t)(oy0 + oyl) * P.out_sh, acc[r], ch, P.epi);
+      if (oyl < nrows) aa_store<true>(P.out, base + (int64_t)oyl * sh, acc[r], ch, P.epi);
     }
   }
 }
 
 }  // namespace
 
-int launch_crops(const aa_image_desc* images, const aa_crop* crops, int32_t count, int32_t dtype, int64_t channels,
-                 int32_t channels_last, const aa_tensor_desc* out, int filter, int align, const OutEpi& epi, cudaStream_t stream,
-                 int32_t* launches) {
+int launch_crops(const char* name, const aa_image_desc* images, const aa_crop_ex* crops, int32_t count, int32_t dtype,
+                 int64_t channels, int32_t channels_last, const aa_tensor_desc* out, int filter, int align, const OutEpi& epi,
+                 cudaStream_t stream, int32_t* launches) {
   const int64_t es = dtype == AA_U8 ? 1 : 4;
   const int Ci = channels_last ? (int)channels : 1;
   const int64_t owf = out->w * Ci;
   const int64_t tiles_x = (owf + TW - 1) / TW, tiles_y = (out->h + TH - 1) / TH;
-  if (tiles_x * tiles_y >= (1ll << 31)) return fail(AA_ERR_UNSUPPORTED, "aa_resize_crops: output too large for one launch");
-  std::unique_ptr<CropParams> hold(new CropParams);  // ~25 KB, kept off the stack; each launch copies it
+  if (tiles_x * tiles_y >= (1ll << 31)) return fail(AA_ERR_UNSUPPORTED, std::string(name) + ": output too large for one launch");
+  std::unique_ptr<CropParams> hold(new CropParams);  // ~28 KB, kept off the stack; each launch copies it
   CropParams& P = *hold;
   P.out = out->data;
   P.epi = epi;
@@ -167,17 +179,18 @@ int launch_crops(const aa_image_desc* images, const aa_crop* crops, int32_t coun
     P.first = first;
     for (int k = 0; k < n; k++) {
       const aa_image_desc& m = images[first + k];
-      const aa_crop& b = crops[first + k];
+      const aa_crop_ex& b = crops[first + k];
       CropDesc& d = P.c[k];
       d.src = (const char*)m.data + (b.top * m.stride_h + b.left * Ci) * es;
       d.stride_h = m.stride_h;
       d.stride_c = channels_last ? 0 : m.stride_c;
       d.h = (int32_t)b.height; d.w = (int32_t)b.width;
-      d.scale_h = host_scale_f32(b.height, out->h, align);
-      d.scale_w = host_scale_f32(b.width, out->w, align);
-      d.kh = (int16_t)host_interp_size(b.height, out->h, filter, align, AA_F32);
-      d.kw = (int16_t)host_interp_size(b.width, out->w, filter, align, AA_F32);
-      d.hflip = b.hflip ? 1 : 0;
+      d.y0 = (int32_t)b.crop_top; d.x0 = (int32_t)b.crop_left;
+      d.scale_h = host_scale_f32(b.height, b.resized_h, align);
+      d.scale_w = host_scale_f32(b.width, b.resized_w, align);
+      d.kh = (int16_t)host_interp_size(b.height, b.resized_h, filter, align, AA_F32);
+      d.kw = (int16_t)host_interp_size(b.width, b.resized_w, filter, align, AA_F32);
+      d.flip = b.flip;
     }
     const dim3 grid((unsigned)(tiles_x * tiles_y), (unsigned)(channels_last ? 1 : channels), (unsigned)n);
     if (dtype == AA_U8) aa_crops_kernel<uint8_t><<<grid, TW * NTY, 0, stream>>>(P);
