@@ -262,6 +262,38 @@ int aa_resize_crops_ex(const aa_image_desc* images, const aa_crop_ex* crops, int
                        int32_t channels_last, const aa_tensor_desc* out, int filter, int align_corners, uint32_t flags,
                        const aa_epilogue* epilogue, void* cuda_stream, int32_t* launches_out);
 
+/* Padded resize-then-crop: aa_resize_crops_ex whose windows may reach past the resized image.  out[i] is the (oH, oW) window
+ * at (crop_top, crop_left) of P_i, flipped as `flip` says, where P_i is R_i of aa_resize_crops_ex extended in every direction
+ * by a constant.  What it reproduces:
+ *   - torchvision v2 center_crop of a crop larger than the image (pad with 0, then crop): AA_FILL_INPUT with 0;
+ *   - letterboxing (resize with the aspect ratio kept, centred on a constant border such as 114): AA_FILL_INPUT;
+ *   - pad-to-batch (resize, place at the top left of a common canvas, pad with zeros after normalisation, as torchvision
+ *     detection's batch_images): AA_FILL_OUTPUT with 0;
+ *   - RandomCrop(size, padding=p, fill=v) + horizontal flip: pad(img, p, v), crop, hflip: AA_FILL_INPUT with the box filter,
+ *     resized size = image size (one tap of weight 1) and a window origin in [-p, p].
+ * Outputs inside R_i are bit-identical to aa_resize_crops_ex.  Outputs outside R_i are bit-identical to aa_resize_forward_ex
+ * of a [1, C, 1, 1] float32 tensor holding value[c], resized to 1x1 with the same out dtype and flags, and with the same
+ * epilogue (AA_FILL_INPUT: value is a pixel of the input, e.g. torchvision's pad fill before Normalize / ToDtype) or with
+ * none (AA_FILL_OUTPUT: value is stored as it is, converted to out->dtype only: f16/bf16 round to nearest, u8 clamps, then
+ * truncates or rounds as AA_FLAG_ROUND_NEAREST says).
+ *   - fill == NULL or mode AA_FILL_NONE: exactly aa_resize_crops_ex (same refusals, same launches);
+ *   - with a fill, a window may overhang any edge of R_i or lie wholly outside it (all fill).  Tiles of the output with no
+ *     output inside R_i store the fill and read nothing; launches, graph capturability and the reads staying inside the box
+ *     are those of aa_resize_crops_ex;
+ *   - AA_ERR_INVALID for an unknown mode; AA_ERR_UNSUPPORTED with a fill for channels > 4 and (message names the crop index)
+ *     for a crop_top, crop_top + oH, crop_left or crop_left + oW outside int32.  Every other check is that of
+ *     aa_resize_crops_ex, the window check excepted; every check happens before the first launch. */
+#define AA_FILL_NONE 0   /* windows must lie inside the resized image: exactly aa_resize_crops_ex */
+#define AA_FILL_INPUT 1  /* value[c] is a pixel value of the input: it goes through the epilogue like a resized value */
+#define AA_FILL_OUTPUT 2 /* value[c] is stored as it is, only converted to out->dtype (zeros after normalisation) */
+typedef struct aa_fill {
+  int32_t mode;
+  float value[4]; /* per channel; channels <= 4 whenever mode != AA_FILL_NONE */
+} aa_fill;
+int aa_resize_crops_pad(const aa_image_desc* images, const aa_crop_ex* crops, int32_t count, int32_t dtype, int64_t channels,
+                        int32_t channels_last, const aa_tensor_desc* out, int filter, int align_corners, uint32_t flags,
+                        const aa_epilogue* epilogue, const aa_fill* fill, void* cuda_stream, int32_t* launches_out);
+
 /* grad_in = Wh^T * grad_out * Ww : the true adjoint of aa_resize_forward, gather form, no atomics,
  * no zero-fill pass.  Replaces ti_upsample_bilinear2d_backward_cpu,
  * aa_interpolation_backward_impl.h:185-219 (linear_backward), whose body is the NON-antialiased

@@ -20,7 +20,7 @@ from ._build_ext import EXT, EXT_NAME, LIB
 
 __all__ = ["load", "linear_forward", "cubic_forward", "nearest_forward", "linear_backward", "cubic_backward",
            "nearest_backward", "linear_backward_nonaa", "forward_with_flags", "resize_to_uint8", "decode_resize_normalize", "resized_crops", "resized_output_size",
-           "resize_center_crop", "five_crop", "ten_crop", "AAResize", "aa_resize", "capi"]
+           "resize_center_crop", "five_crop", "ten_crop", "resize_pad_batch", "AAResize", "aa_resize", "capi"]
 
 _ext = None
 
@@ -197,21 +197,24 @@ def _crop_hw(crop_size):
     return crop_size[0], crop_size[1]
 
 
-def _eval_crops(hw, size, crop_size, kind, vertical_flip=False, max_size=None):
+def _eval_crops(hw, size, crop_size, kind, vertical_flip=False, max_size=None, pad=False):
     """Host-only: the aa_crop_ex rows ([N, kinds] of capi.crop_ex_dtype) of Resize(size, max_size) followed by
-    CenterCrop ("center"), FiveCrop ("five") or TenCrop ("ten") of crop_size, for images of sizes hw ([N, 2]: h, w)."""
+    CenterCrop ("center"), FiveCrop ("five") or TenCrop ("ten") of crop_size, for images of sizes hw ([N, 2]: h, w).
+    pad (CenterCrop only): a crop larger than the resized image gets the window torchvision's zero padding gives."""
     import numpy as np
     ch, cw = _crop_hw(crop_size)
     hw = np.asarray(hw, np.int64).reshape(-1, 2)
     R = np.array([resized_output_size(int(h), int(w), size, max_size) for h, w in hw], np.int64).reshape(-1, 2)
     small = np.nonzero((R[:, 0] < ch) | (R[:, 1] < cw))[0]
-    if len(small):
+    if len(small) and not (pad and kind == "center"):
         i = int(small[0])
         raise ValueError(f"crop size {(ch, cw)} is larger than the resized image {tuple(int(v) for v in R[i])} of image {i}: "
                          "zero padding is not supported")
     dy, dx = R[:, 0] - ch, R[:, 1] - cw
     # torchvision's anchor int(round(d / 2.0)): Python's round, half to even, which np.round also does
     cy, cx = np.round(dy / 2.0).astype(np.int64), np.round(dx / 2.0).astype(np.int64)
+    # v2 center_crop pads a too small axis by (c - R) // 2 before and (c - R + 1) // 2 after, then crops at 0 on it
+    cy, cx = np.where(dy < 0, -((-dy) // 2), cy), np.where(dx < 0, -((-dx) // 2), cx)
     z = np.zeros_like(dy)
     five = [(z, z, 0), (z, dx, 0), (dy, z, 0), (dy, dx, 0), (cy, cx, 0)]  # torchvision's order: tl, tr, bl, br, center
     if kind == "center":
@@ -231,30 +234,38 @@ def _eval_crops(hw, size, crop_size, kind, vertical_flip=False, max_size=None):
     return crops
 
 
-def _resize_then_crop(images, size, crop_size, kind, vertical_flip, mode, max_size, mean, std, out_dtype):
-    """_eval_crops of every image in one aa_resize_crops_ex call (ceil(crops / 512) launches) -> [N * kinds, C, ch, cw]."""
+def _resize_then_crop(images, size, crop_size, kind, vertical_flip, mode, max_size, mean, std, out_dtype, pad=False):
+    """_eval_crops of every image in one aa_resize_crops_ex call, or one aa_resize_crops_pad call with a zero input fill when
+    pad (ceil(crops / 512) launches) -> [N * kinds, C, ch, cw]."""
     import numpy as np
     import torch
     images = _image_list(images)
     hwc = capi._is_hwc(images[0])
     C = images[0].shape[-1] if hwc else images[0].shape[0]
     hw = [(t.shape[0], t.shape[1]) if hwc else (t.shape[1], t.shape[2]) for t in images]
-    crops = _eval_crops(hw, size, crop_size, kind, vertical_flip, max_size)
+    crops = _eval_crops(hw, size, crop_size, kind, vertical_flip, max_size, pad)
     scale, bias, out_dtype, flags = _normalize_args(mean, std, out_dtype)
     ch, cw = _crop_hw(crop_size)
     out = torch.empty((crops.size, C, ch, cw), dtype=out_dtype, device=images[0].device)
     rows = np.repeat(capi.image_descs(images, hwc), crops.shape[1])
-    capi.launch_crops_ex(rows, crops.reshape(-1), capi._dtype_code(images[0]), C, hwc, out, mode, scale, bias, flags=flags)
+    if pad:
+        capi.launch_crops_pad(rows, crops.reshape(-1), capi._dtype_code(images[0]), C, hwc, out, mode, capi.FILL_INPUT, 0.0,
+                              scale, bias, flags=flags)
+    else:
+        capi.launch_crops_ex(rows, crops.reshape(-1), capi._dtype_code(images[0]), C, hwc, out, mode, scale, bias, flags=flags)
     return out
 
 
-def resize_center_crop(images, size, crop_size, mode="bilinear", max_size=None, mean=None, std=None, out_dtype=None):
+def resize_center_crop(images, size, crop_size, mode="bilinear", max_size=None, mean=None, std=None, out_dtype=None,
+                       pad=False):
     """The evaluation transform CenterCrop(crop_size)(Resize(size, antialias=True, max_size=max_size)(img)) of a batch in
     one kernel launch: every image resized with its own aspect ratio (resized_output_size), then the centre window at
     torchvision's anchor int(round((R - c) / 2.0)) stored; only the window's outputs are computed.  images, mode, mean/std
-    and out_dtype as in resized_crops.  A crop larger than a resized image raises ValueError (torchvision would zero-pad).
+    and out_dtype as in resized_crops.  A crop larger than a resized image raises ValueError unless pad=True, which
+    zero-pads it as torchvision v2 center_crop does: (c - R) // 2 zeros before and (c - R + 1) // 2 after on each axis that
+    is too small, zeros of the input (they go through mean/std like pixels), still in one launch.
     Returns a contiguous [N,C,ch,cw] tensor."""
-    return _resize_then_crop(images, size, crop_size, "center", False, mode, max_size, mean, std, out_dtype)
+    return _resize_then_crop(images, size, crop_size, "center", False, mode, max_size, mean, std, out_dtype, pad)
 
 
 def five_crop(images, size, crop_size, mode="bilinear", max_size=None, mean=None, std=None, out_dtype=None):
@@ -275,6 +286,77 @@ def ten_crop(images, size, crop_size, vertical_flip=False, mode="bilinear", max_
     vertical flip likewise).  Other arguments as in resize_center_crop."""
     y = _resize_then_crop(images, size, crop_size, "ten", vertical_flip, mode, max_size, mean, std, out_dtype)
     return y.view(-1, 10, *y.shape[1:])
+
+
+def _pad_layout(hw, size, max_size=None, size_divisible=32, canvas=None, align="top_left"):
+    """Host-only: (resized sizes [N, 2], canvas (Hc, Wc), placements [N, 4] as (top, left, h, w)) of resize_pad_batch."""
+    import numpy as np
+    hw = np.asarray(hw, np.int64).reshape(-1, 2)
+    per_image = size is not None and not isinstance(size, numbers.Integral) and len(size) > 0 and \
+        not isinstance(size[0], numbers.Integral)
+    if per_image:
+        R = np.asarray([[int(v) for v in s] for s in size], np.int64).reshape(-1, 2)
+        if len(R) != len(hw):
+            raise ValueError(f"resize_pad_batch: {len(R)} sizes for {len(hw)} images")
+        if (R < 1).any():
+            raise ValueError("resize_pad_batch: every resized size must be at least 1x1")
+    else:
+        R = np.array([resized_output_size(int(h), int(w), size, max_size) for h, w in hw], np.int64).reshape(-1, 2)
+    if canvas is None:
+        d = int(size_divisible or 1)
+        Hc, Wc = (int(-(-int(R[:, k].max()) // d) * d) for k in (0, 1))
+    else:
+        Hc, Wc = _crop_hw(canvas)
+        big = np.nonzero((R[:, 0] > Hc) | (R[:, 1] > Wc))[0]
+        if len(big):
+            i = int(big[0])
+            raise ValueError(f"resized image {tuple(int(v) for v in R[i])} of image {i} is larger than the canvas {(Hc, Wc)}")
+    if align == "top_left":
+        top, left = np.zeros(len(R), np.int64), np.zeros(len(R), np.int64)
+    elif align == "center":
+        top, left = (Hc - R[:, 0]) // 2, (Wc - R[:, 1]) // 2
+    else:
+        raise ValueError(f"align must be 'top_left' or 'center', got {align!r}")
+    return R, (Hc, Wc), np.stack([top, left, R[:, 0], R[:, 1]], axis=1)
+
+
+def resize_pad_batch(images, size, max_size=None, size_divisible=32, canvas=None, align="top_left", fill=None, pad_value=None,
+                     mode="bilinear", mean=None, std=None, out_dtype=None):
+    """Variable-size images -> one padded batch in one kernel launch per 512 images: each image resized with torchvision v2
+    `resize(img, size, max_size=max_size, antialias=True)` (not the non-antialiased resize of torchvision's detection
+    transform) and placed on a common canvas whose other outputs hold a constant.  Letterboxing is
+    canvas=(640, 640), align="center", fill=114; pad-to-batch (torchvision detection's batch_images, DETR's nested tensors)
+    is the default: the canvas is the largest resized size rounded up to size_divisible, images at the top left, zeros
+    after normalisation.
+
+    images: as in resized_crops.
+    size:   what resized_output_size takes, or one (h, w) per image for a caller with its own size rule.
+    canvas: None (see above) or a fixed (H, W); an image resized larger than it raises ValueError.
+    align:  "top_left", or "center" with offsets ((Hc - h) // 2, (Wc - w) // 2).
+    fill / pad_value: the constant, one number or one per channel; at most one of them may be given.  fill is a pixel value
+            of the input and goes through mean/std like a pixel; pad_value is stored as it is.  The default is pad_value=0.
+    mean/std/out_dtype: as in resized_crops.
+    Returns (batch [N, C, Hc, Wc] contiguous, placements): placements is an int64 CPU tensor [N, 4] with (top, left, h, w)
+    of each resized image in the canvas, what a caller needs to map boxes and to build masks."""
+    import numpy as np
+    import torch
+    if fill is not None and pad_value is not None:
+        raise ValueError("resize_pad_batch: give fill or pad_value, not both")
+    fill_mode, value = (capi.FILL_INPUT, fill) if fill is not None else (capi.FILL_OUTPUT, 0.0 if pad_value is None else pad_value)
+    images = _image_list(images)
+    hwc = capi._is_hwc(images[0])
+    C = images[0].shape[-1] if hwc else images[0].shape[0]
+    hw = [(t.shape[0], t.shape[1]) if hwc else (t.shape[1], t.shape[2]) for t in images]
+    R, (Hc, Wc), place = _pad_layout(hw, size, max_size, size_divisible, canvas, align)
+    crops = np.zeros(len(R), capi.crop_ex_dtype())
+    crops["height"], crops["width"] = [h for h, _ in hw], [w for _, w in hw]
+    crops["resized_h"], crops["resized_w"] = R[:, 0], R[:, 1]
+    crops["crop_top"], crops["crop_left"] = -place[:, 0], -place[:, 1]
+    scale, bias, out_dtype, flags = _normalize_args(mean, std, out_dtype)
+    out = torch.empty((len(R), C, Hc, Wc), dtype=out_dtype, device=images[0].device)
+    capi.launch_crops_pad(capi.image_descs(images, hwc), crops, capi._dtype_code(images[0]), C, hwc, out, mode, fill_mode, value,
+                          scale, bias, flags=flags)
+    return out, torch.from_numpy(place)
 
 
 from .functional import AAResize, aa_resize  # noqa: E402

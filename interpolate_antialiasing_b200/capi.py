@@ -15,11 +15,12 @@ FLAG_AUTO, FLAG_FORCE_GENERAL, FLAG_FORCE_STREAM, FLAG_STREAM_TMA, FLAG_STREAM_L
 FLAG_VMMA = 64
 FLAG_STRICT_NONFINITE = 128
 FLAG_ASSUME_FINITE = 256  # skip the drain launch behind the fast float kernels (csrc/aa_redo.cu)
+FILL_NONE, FILL_INPUT, FILL_OUTPUT = 0, 1, 2  # aa_fill modes of aa_resize_crops_pad
 FILTERS = {"nearest": BOX, "box": BOX, "bilinear": TRIANGLE, "linear": TRIANGLE, "bicubic": CUBIC, "cubic": CUBIC}
 
 EXPORTS = [
     "aa_abi_version", "aa_last_error", "aa_interp_size", "aa_host_tables", "aa_build_tables", "aa_build_tables_sf", "aa_warm_tables",
-    "aa_clear_table_cache", "aa_check_device", "aa_debug_counters", "aa_resize_forward", "aa_resize_forward_sf", "aa_resize_backward_sf", "aa_resize_forward_ex", "aa_resize_forward_ragged", "aa_resize_crops", "aa_resize_crops_ex", "aa_resize_backward",
+    "aa_clear_table_cache", "aa_check_device", "aa_debug_counters", "aa_resize_forward", "aa_resize_forward_sf", "aa_resize_backward_sf", "aa_resize_forward_ex", "aa_resize_forward_ragged", "aa_resize_crops", "aa_resize_crops_ex", "aa_resize_crops_pad", "aa_resize_backward",
     "aa_resize_backward_nonaa_bilinear", "aa_resize_forward_host", "aa_resize_forward_host_multi", "aa_launch_count",
 ]
 
@@ -57,6 +58,12 @@ class CropEx(ctypes.Structure):
     _fields_ = [("top", ctypes.c_int64), ("left", ctypes.c_int64), ("height", ctypes.c_int64), ("width", ctypes.c_int64),
                 ("resized_h", ctypes.c_int64), ("resized_w", ctypes.c_int64), ("crop_top", ctypes.c_int64),
                 ("crop_left", ctypes.c_int64), ("flip", ctypes.c_int32)]
+
+
+class Fill(ctypes.Structure):
+    """aa_fill: how aa_resize_crops_pad fills outputs outside the resized image (FILL_NONE, FILL_INPUT: a pixel value of the
+    input that goes through the epilogue, FILL_OUTPUT: a value stored as it is) and the value per channel."""
+    _fields_ = [("mode", ctypes.c_int32), ("value", ctypes.c_float * 4)]
 
 
 def crop_ex_dtype():
@@ -108,6 +115,8 @@ def lib():
         L.aa_resize_forward_ragged.argtypes = [P(ImageDesc), i32, i32, i64, i32, P(TensorDesc), i32, i32, u32, P(Epilogue), vp, P(i32)]
         L.aa_resize_crops.argtypes = [P(ImageDesc), P(Crop), i32, i32, i64, i32, P(TensorDesc), i32, i32, u32, P(Epilogue), vp, P(i32)]
         L.aa_resize_crops_ex.argtypes = [vp, vp, i32, i32, i64, i32, P(TensorDesc), i32, i32, u32, P(Epilogue), vp, P(i32)]
+        L.aa_resize_crops_pad.argtypes = [vp, vp, i32, i32, i64, i32, P(TensorDesc), i32, i32, u32, P(Epilogue), P(Fill), vp,
+                                          P(i32)]
         L.aa_resize_backward.argtypes = [P(TensorDesc), P(TensorDesc), i32, i32, u32, vp]
         L.aa_resize_backward_nonaa_bilinear.argtypes = [P(TensorDesc), P(TensorDesc), i32, vp]
         L.aa_resize_forward_host.argtypes = [P(TensorDesc), P(TensorDesc), i32, i32, u32]
@@ -371,6 +380,60 @@ def resize_crops_ex(images, crops, output_size, filter, out=None, scale=None, bi
         out = torch.empty((n, C, oH, oW), dtype=torch.float32, device=images[0].device)
     dtype = _dtype_code(images[0]) if n else F32
     return out, launch_crops_ex(image_descs(images, hwc), rows, dtype, C, hwc, out, filter, scale, bias, align_corners, flags)
+
+
+def fill_struct(mode, value):
+    """Fill of `mode` with `value`: a number for every channel or one number per channel (at most 4)."""
+    f = Fill()
+    f.mode = int(mode)
+    v = [float(value)] * 4 if isinstance(value, (int, float)) else [float(t) for t in value]
+    if not 1 <= len(v) <= 4:
+        raise ValueError(f"fill value: one number or one per channel (at most 4), got {value}")
+    v = v * 4 if len(v) == 1 else v + [0.0] * (4 - len(v))
+    for i in range(4):
+        f.value[i] = v[i]
+    return f
+
+
+def launch_crops_pad(image_rows, crop_rows, dtype, channels, hwc, out, filter, fill_mode, fill_value, scale=None, bias=None,
+                     align_corners=False, flags=FLAG_AUTO):
+    """aa_resize_crops_pad on descriptor arrays (as launch_crops_ex) with the fill (fill_mode, fill_value); -> launches."""
+    assert len(image_rows) == len(crop_rows) and image_rows.dtype == image_desc_dtype() and crop_rows.dtype == crop_ex_dtype()
+    assert image_rows.flags.c_contiguous and crop_rows.flags.c_contiguous
+    e = _epilogue(scale, bias)
+    f = fill_struct(fill_mode, fill_value)
+    k = ctypes.c_int32(0)
+    do = desc(out)
+    check(lib().aa_resize_crops_pad(image_rows.ctypes.data, crop_rows.ctypes.data, len(crop_rows), dtype, channels, int(hwc),
+                                    ctypes.byref(do), _filter(filter), int(align_corners), flags, ctypes.byref(e),
+                                    ctypes.byref(f), _stream(out), ctypes.byref(k)))
+    return k.value
+
+
+def resize_crops_pad(images, crops, output_size, filter, fill=0.0, fill_mode=FILL_INPUT, out=None, scale=None, bias=None,
+                     align_corners=False, flags=FLAG_AUTO):
+    """Padded resize-then-crop (aa_resize_crops_pad): resize_crops_ex whose windows may reach past the resized image (a
+    negative crop_top / crop_left, or past its end); outputs there store `fill` (one number, or one per channel), as a
+    pixel value of the input (FILL_INPUT) or as it is (FILL_OUTPUT).  Arguments as in resize_crops_ex.
+    Returns (out, launches)."""
+    import torch
+    n = len(images)
+    rows = crop_ex_array(crops)
+    if len(rows) != n:
+        raise ValueError("resize_crops_pad: images and crops must have the same length")
+    hwc = bool(n) and _is_hwc(images[0])
+    if n:
+        C = images[0].shape[-1] if hwc else images[0].shape[0]
+    elif out is not None:
+        C = out.shape[1]
+    else:
+        raise ValueError("resize_crops_pad: an empty batch needs `out`")
+    oH, oW = int(output_size[0]), int(output_size[1])
+    if out is None:
+        out = torch.empty((n, C, oH, oW), dtype=torch.float32, device=images[0].device)
+    dtype = _dtype_code(images[0]) if n else F32
+    return out, launch_crops_pad(image_descs(images, hwc), rows, dtype, C, hwc, out, filter, fill_mode, fill, scale, bias,
+                                 align_corners, flags)
 
 
 def resize_backward(grad_out, input_size, filter, align_corners=False, nonaa=False, flags=FLAG_AUTO, scales=None, out=None):

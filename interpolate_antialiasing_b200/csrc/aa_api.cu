@@ -452,13 +452,14 @@ int aa_resize_forward_ragged(const aa_image_desc* images, int32_t count, int32_t
 }
 
 static_assert(sizeof(aa_crop_ex) == 72, "aa_crop_ex layout (capi.CropEx and capi.crop_ex_dtype() mirror it)");
+static_assert(sizeof(aa_fill) == 20, "aa_fill layout (capi.Fill mirrors it)");
 
-// aa_resize_crops and aa_resize_crops_ex: every check before the first launch, then the crops kernel.  `name` prefixes
-// the messages.
+// aa_resize_crops, aa_resize_crops_ex and aa_resize_crops_pad: every check before the first launch, then the crops kernel.
+// `name` prefixes the messages.  With a fill (mode != AA_FILL_NONE) a window may lie anywhere its edges fit in int32.
 static int resize_crops_impl(const char* name, const aa_image_desc* images, const aa_crop_ex* crops, int32_t count,
                              int32_t dtype, int64_t channels, int32_t channels_last, const aa_tensor_desc* out, int filter,
-                             int align_corners, uint32_t flags, const aa_epilogue* epilogue, void* cuda_stream,
-                             int32_t* launches_out) {
+                             int align_corners, uint32_t flags, const aa_epilogue* epilogue, const aa_fill* fill,
+                             void* cuda_stream, int32_t* launches_out) {
   int rc;
   const std::string nm = name;
   if (launches_out) *launches_out = 0;
@@ -474,6 +475,10 @@ static int resize_crops_impl(const char* name, const aa_image_desc* images, cons
   const int64_t ci = channels_last ? channels : 1;
   if (out->h >= (1ll << 31) || out->w * ci >= (1ll << 31)) return fail(AA_ERR_UNSUPPORTED, nm + ": output plane too large");
   if (!channels_last && channels > 65535) return fail(AA_ERR_UNSUPPORTED, nm + ": more than 65535 planar channels");
+  if (fill && fill->mode != AA_FILL_NONE && fill->mode != AA_FILL_INPUT && fill->mode != AA_FILL_OUTPUT)
+    return fail(AA_ERR_INVALID, nm + ": unknown fill mode " + std::to_string(fill->mode));
+  const bool padded = fill && fill->mode != AA_FILL_NONE;
+  if (padded && channels > 4) return fail(AA_ERR_UNSUPPORTED, nm + ": a fill takes at most 4 channels");
   OutEpi epi;
   epi.round = (flags & AA_FLAG_ROUND_NEAREST) ? 1 : 0;
   switch (out->dtype) {
@@ -507,7 +512,13 @@ static int resize_crops_impl(const char* name, const aa_image_desc* images, cons
     if (b.resized_h < 1 || b.resized_w < 1)
       return fail(AA_ERR_INVALID, at + ": resized size " + std::to_string(b.resized_h) + "x" + std::to_string(b.resized_w) +
                                       " is empty");
-    if (b.crop_top < 0 || b.crop_left < 0 || b.crop_top > b.resized_h - out->h || b.crop_left > b.resized_w - out->w)
+    if (padded) {
+      const int64_t lo = INT32_MIN, hi = INT32_MAX;
+      if (b.crop_top < lo || b.crop_top > hi - out->h || b.crop_left < lo || b.crop_left > hi - out->w)
+        return fail(AA_ERR_UNSUPPORTED, at + ": window (top " + std::to_string(b.crop_top) + ", left " +
+                                            std::to_string(b.crop_left) + ", " + std::to_string(out->h) + "x" +
+                                            std::to_string(out->w) + ") has an edge outside int32");
+    } else if (b.crop_top < 0 || b.crop_left < 0 || b.crop_top > b.resized_h - out->h || b.crop_left > b.resized_w - out->w)
       return fail(AA_ERR_INVALID, at + ": window (top " + std::to_string(b.crop_top) + ", left " + std::to_string(b.crop_left) +
                                       ", " + std::to_string(out->h) + "x" + std::to_string(out->w) + ") is not inside the " +
                                       std::to_string(b.resized_h) + "x" + std::to_string(b.resized_w) + " resized image");
@@ -523,7 +534,7 @@ static int resize_crops_impl(const char* name, const aa_image_desc* images, cons
   if (!g.ok) return cuda_fail(g.err, "cudaSetDevice");
   int32_t launches = 0;
   rc = launch_crops(name, images, crops, count, dtype, channels, channels_last, out, filter, align_corners ? 1 : 0, epi,
-                    (cudaStream_t)cuda_stream, &launches);
+                    fill, (cudaStream_t)cuda_stream, &launches);
   if (launches_out) *launches_out = launches;
   return rc;
 }
@@ -532,7 +543,14 @@ int aa_resize_crops_ex(const aa_image_desc* images, const aa_crop_ex* crops, int
                        int32_t channels_last, const aa_tensor_desc* out, int filter, int align_corners, uint32_t flags,
                        const aa_epilogue* epilogue, void* cuda_stream, int32_t* launches_out) {
   return resize_crops_impl("aa_resize_crops_ex", images, crops, count, dtype, channels, channels_last, out, filter,
-                           align_corners, flags, epilogue, cuda_stream, launches_out);
+                           align_corners, flags, epilogue, nullptr, cuda_stream, launches_out);
+}
+
+int aa_resize_crops_pad(const aa_image_desc* images, const aa_crop_ex* crops, int32_t count, int32_t dtype, int64_t channels,
+                        int32_t channels_last, const aa_tensor_desc* out, int filter, int align_corners, uint32_t flags,
+                        const aa_epilogue* epilogue, const aa_fill* fill, void* cuda_stream, int32_t* launches_out) {
+  return resize_crops_impl("aa_resize_crops_pad", images, crops, count, dtype, channels, channels_last, out, filter,
+                           align_corners, flags, epilogue, fill, cuda_stream, launches_out);
 }
 
 int aa_resize_crops(const aa_image_desc* images, const aa_crop* crops, int32_t count, int32_t dtype, int64_t channels,
@@ -545,7 +563,7 @@ int aa_resize_crops(const aa_image_desc* images, const aa_crop* crops, int32_t c
     ex[i] = aa_crop_ex{b.top, b.left, b.height, b.width, out ? out->h : 0, out ? out->w : 0, 0, 0, b.hflip ? 1 : 0};
   }
   return resize_crops_impl("aa_resize_crops", images, crops ? ex.data() : nullptr, count, dtype, channels, channels_last, out,
-                           filter, align_corners, flags, epilogue, cuda_stream, launches_out);
+                           filter, align_corners, flags, epilogue, nullptr, cuda_stream, launches_out);
 }
 
 static int backward_impl(const aa_tensor_desc* gout, const aa_tensor_desc* gin, int filter, int align_corners, uint32_t flags,

@@ -412,14 +412,15 @@ int vmma_read_counters(int device, unsigned long long* out, int reset);
 int vmma_warm(AxisTables* th, cudaStream_t stream);  // everything a later launch_vmma would allocate or synchronise for
 void vmma_plan_clear();
 
-// Batched resized crops (aa_crops.cu): arguments validated by aa_resize_crops / aa_resize_crops_ex (`name` prefixes the
-// messages); ceil(count / kCropsPerLaunch) launches, counted into *launches.  The per-crop descriptors travel in the kernel
-// parameters (56 bytes each).
+// Batched resized crops (aa_crops.cu): arguments validated by aa_resize_crops / aa_resize_crops_ex / aa_resize_crops_pad
+// (`name` prefixes the messages); ceil(count / kCropsPerLaunch) launches, counted into *launches.  The per-crop descriptors
+// travel in the kernel parameters (56 bytes each).  `fill` NULL or AA_FILL_NONE: windows inside the resized images;
+// otherwise the padded kernel variant.
 constexpr int kCropsPerLaunch = 512;
 constexpr int kCropMaxTaps = 65;  // largest interp_size (2*ceil(support)+1) of a crop axis: shared weight rows
 int launch_crops(const char* name, const aa_image_desc* images, const aa_crop_ex* crops, int32_t count, int32_t dtype,
                  int64_t channels, int32_t channels_last, const aa_tensor_desc* out, int filter, int align, const OutEpi& epi,
-                 cudaStream_t stream, int32_t* launches);
+                 const aa_fill* fill, cudaStream_t stream, int32_t* launches);
 
 int launch_backward_nonaa(const void* gout, void* gin, int dtype, const Layout& lout, const Layout& lin,
                           int64_t oH, int64_t oW, int64_t H, int64_t W, int align, cudaStream_t stream);
