@@ -103,14 +103,18 @@ def decode_resize_normalize(x_hwc_u8, output_size, mean, std, mode="bilinear", o
     return capi.resize_forward_ex(x, output_size, mode, out, scale, bias, align_corners)
 
 
-def _image_list(images):
-    """The `images` argument of resized_crops and the eval-crop helpers as a list of 3-D CUDA tensors."""
+def _image_batch(images):
+    """The `images` argument of resized_crops and the eval-crop helpers -> (list of 3-D CUDA tensors, hwc, channels,
+    [(h, w)] per image)."""
     import torch
     if torch.is_tensor(images):
         assert images.dim() == 4 and images.is_cuda
         cl = images.is_contiguous(memory_format=torch.channels_last) and not images.is_contiguous()
         images = [t.permute(1, 2, 0) if cl else t for t in images.unbind(0)]
-    return images
+    hwc = capi._is_hwc(images[0])
+    C = images[0].shape[-1] if hwc else images[0].shape[0]
+    hw = [(t.shape[0], t.shape[1]) if hwc else (t.shape[1], t.shape[2]) for t in images]
+    return images, hwc, C, hw
 
 
 def _normalize_args(mean, std, out_dtype):
@@ -139,14 +143,12 @@ def resized_crops(images, boxes, size, mode="bilinear", hflip=None, mean=None, s
             out_dtype=torch.uint8.
     Returns a contiguous [N,C,oH,oW] tensor."""
     import torch
-    images = _image_list(images)
+    images, _, C, _ = _image_batch(images)
     if isinstance(boxes, torch.Tensor):
         boxes = boxes.tolist()
     if hflip is not None and isinstance(hflip, torch.Tensor):
         hflip = hflip.tolist()
     oH, oW = (int(size), int(size)) if isinstance(size, int) else (int(size[0]), int(size[1]))
-    hwc = capi._is_hwc(images[0])
-    C = images[0].shape[-1] if hwc else images[0].shape[0]
     scale, bias, out_dtype, flags = _normalize_args(mean, std, out_dtype)
     out = torch.empty((len(images), C, oH, oW), dtype=out_dtype, device=images[0].device)
     return capi.resize_crops(images, boxes, (oH, oW), mode, out=out, hflip=hflip, scale=scale, bias=bias,
@@ -239,20 +241,14 @@ def _resize_then_crop(images, size, crop_size, kind, vertical_flip, mode, max_si
     pad (ceil(crops / 512) launches) -> [N * kinds, C, ch, cw]."""
     import numpy as np
     import torch
-    images = _image_list(images)
-    hwc = capi._is_hwc(images[0])
-    C = images[0].shape[-1] if hwc else images[0].shape[0]
-    hw = [(t.shape[0], t.shape[1]) if hwc else (t.shape[1], t.shape[2]) for t in images]
+    images, hwc, C, hw = _image_batch(images)
     crops = _eval_crops(hw, size, crop_size, kind, vertical_flip, max_size, pad)
     scale, bias, out_dtype, flags = _normalize_args(mean, std, out_dtype)
     ch, cw = _crop_hw(crop_size)
     out = torch.empty((crops.size, C, ch, cw), dtype=out_dtype, device=images[0].device)
     rows = np.repeat(capi.image_descs(images, hwc), crops.shape[1])
-    if pad:
-        capi.launch_crops_pad(rows, crops.reshape(-1), capi._dtype_code(images[0]), C, hwc, out, mode, capi.FILL_INPUT, 0.0,
-                              scale, bias, flags=flags)
-    else:
-        capi.launch_crops_ex(rows, crops.reshape(-1), capi._dtype_code(images[0]), C, hwc, out, mode, scale, bias, flags=flags)
+    capi.launch_crops(rows, crops.reshape(-1), capi._dtype_code(images[0]), C, hwc, out, mode, scale, bias, flags=flags,
+                      fill=(capi.FILL_INPUT, 0.0) if pad else None)
     return out
 
 
@@ -343,10 +339,7 @@ def resize_pad_batch(images, size, max_size=None, size_divisible=32, canvas=None
     if fill is not None and pad_value is not None:
         raise ValueError("resize_pad_batch: give fill or pad_value, not both")
     fill_mode, value = (capi.FILL_INPUT, fill) if fill is not None else (capi.FILL_OUTPUT, 0.0 if pad_value is None else pad_value)
-    images = _image_list(images)
-    hwc = capi._is_hwc(images[0])
-    C = images[0].shape[-1] if hwc else images[0].shape[0]
-    hw = [(t.shape[0], t.shape[1]) if hwc else (t.shape[1], t.shape[2]) for t in images]
+    images, hwc, C, hw = _image_batch(images)
     R, (Hc, Wc), place = _pad_layout(hw, size, max_size, size_divisible, canvas, align)
     crops = np.zeros(len(R), capi.crop_ex_dtype())
     crops["height"], crops["width"] = [h for h, _ in hw], [w for _, w in hw]
@@ -354,8 +347,8 @@ def resize_pad_batch(images, size, max_size=None, size_divisible=32, canvas=None
     crops["crop_top"], crops["crop_left"] = -place[:, 0], -place[:, 1]
     scale, bias, out_dtype, flags = _normalize_args(mean, std, out_dtype)
     out = torch.empty((len(R), C, Hc, Wc), dtype=out_dtype, device=images[0].device)
-    capi.launch_crops_pad(capi.image_descs(images, hwc), crops, capi._dtype_code(images[0]), C, hwc, out, mode, fill_mode, value,
-                          scale, bias, flags=flags)
+    capi.launch_crops(capi.image_descs(images, hwc), crops, capi._dtype_code(images[0]), C, hwc, out, mode, scale, bias,
+                      flags=flags, fill=(fill_mode, value))
     return out, torch.from_numpy(place)
 
 

@@ -70,14 +70,13 @@ def crop_ex_dtype():
     """numpy structured dtype laid out as aa_crop_ex (72 bytes): an array of it is passed to the C ABI as it stands, so a
     batch of thousands of crops needs no ctypes object per crop."""
     import numpy as np
-    return np.dtype([(f, np.int64) for f, _ in CropEx._fields_[:-1]] + [("flip", np.int32)], align=True)
+    return np.dtype(CropEx)
 
 
 def image_desc_dtype():
     """numpy structured dtype laid out as aa_image_desc (40 bytes)."""
     import numpy as np
-    return np.dtype([("data", np.uint64), ("h", np.int64), ("w", np.int64), ("stride_h", np.int64), ("stride_c", np.int64)],
-                    align=True)
+    return np.dtype(ImageDesc)
 
 
 class Scales(ctypes.Structure):
@@ -112,8 +111,8 @@ def lib():
         L.aa_resize_forward_sf.argtypes = [P(TensorDesc), P(TensorDesc), i32, i32, P(Scales), u32, vp]
         L.aa_resize_backward_sf.argtypes = [P(TensorDesc), P(TensorDesc), i32, i32, P(Scales), u32, vp]
         L.aa_resize_forward_ex.argtypes = [P(TensorDesc), P(TensorDesc), i32, i32, u32, P(Epilogue), vp]
-        L.aa_resize_forward_ragged.argtypes = [P(ImageDesc), i32, i32, i64, i32, P(TensorDesc), i32, i32, u32, P(Epilogue), vp, P(i32)]
-        L.aa_resize_crops.argtypes = [P(ImageDesc), P(Crop), i32, i32, i64, i32, P(TensorDesc), i32, i32, u32, P(Epilogue), vp, P(i32)]
+        L.aa_resize_forward_ragged.argtypes = [vp, i32, i32, i64, i32, P(TensorDesc), i32, i32, u32, P(Epilogue), vp, P(i32)]
+        L.aa_resize_crops.argtypes = [vp, vp, i32, i32, i64, i32, P(TensorDesc), i32, i32, u32, P(Epilogue), vp, P(i32)]
         L.aa_resize_crops_ex.argtypes = [vp, vp, i32, i32, i64, i32, P(TensorDesc), i32, i32, u32, P(Epilogue), vp, P(i32)]
         L.aa_resize_crops_pad.argtypes = [vp, vp, i32, i32, i64, i32, P(TensorDesc), i32, i32, u32, P(Epilogue), P(Fill), vp,
                                           P(i32)]
@@ -220,11 +219,7 @@ def resize_forward(x, output_size, filter, align_corners=False, flags=FLAG_AUTO,
 def resize_forward_ex(x, output_size, filter, out, scale=None, bias=None, align_corners=False, flags=FLAG_AUTO):
     """C-ABI forward with the decode-adjacent epilogue: `out` may be f16/bf16/f32/u8 and channels_first for a
     channels_last `x`; scale/bias (per channel, <= 4) apply v*scale[c] + bias[c] at the store."""
-    e = Epilogue()
-    e.normalize = 1 if scale is not None else 0
-    for i in range(4):
-        e.scale[i] = float(scale[i]) if scale is not None and i < len(scale) else 1.0
-        e.bias[i] = float(bias[i]) if bias is not None and i < len(bias) else 0.0
+    e = _epilogue(scale, bias)
     di, do = desc(x), desc(out)
     check(lib().aa_resize_forward_ex(ctypes.byref(di), ctypes.byref(do), _filter(filter), int(align_corners), flags,
                                      ctypes.byref(e), _stream(x)))
@@ -256,28 +251,35 @@ def resize_forward_ragged(images, output_size, filter, out=None, align_corners=F
     if out is None:
         out = torch.empty((len(images), C, oH, oW), dtype=torch.float32, device=images[0].device,
                           memory_format=torch.channels_last if hwc else torch.contiguous_format)
-    arr = (ImageDesc * len(images))()
-    for i, t in enumerate(images):
-        if hwc:
-            arr[i] = ImageDesc(t.data_ptr(), t.shape[0], t.shape[1], t.stride(0), 1)
-        else:
-            arr[i] = ImageDesc(t.data_ptr(), t.shape[1], t.shape[2], t.stride(1), t.stride(0))
+    rows = image_descs(images, hwc)
+    # an (empty) epilogue is what lets the call store f16/bf16, or planar output from HWC input
     e = None
-    if scale is not None:
-        e = Epilogue()
-        e.normalize = 1
-        for i in range(4):
-            e.scale[i] = float(scale[i]) if i < len(scale) else 1.0
-            e.bias[i] = float(bias[i]) if bias is not None and i < len(bias) else 0.0
-    elif out.dtype in (torch.float16, torch.bfloat16) or (hwc and out.is_contiguous() and C > 1):
-        e = Epilogue()
-        e.normalize = 0
+    if scale is not None or out.dtype in (torch.float16, torch.bfloat16) or (hwc and out.is_contiguous() and C > 1):
+        e = _epilogue(scale, bias)
     n = ctypes.c_int32(0)
     do = desc(out)
-    check(lib().aa_resize_forward_ragged(arr, len(images), _dtype_code(images[0]), C, int(hwc), ctypes.byref(do), _filter(filter),
-                                         int(align_corners), flags, ctypes.byref(e) if e is not None else None, _stream(out),
-                                         ctypes.byref(n)))
+    check(lib().aa_resize_forward_ragged(rows.ctypes.data, len(images), _dtype_code(images[0]), C, int(hwc), ctypes.byref(do),
+                                         _filter(filter), int(align_corners), flags, ctypes.byref(e) if e is not None else None,
+                                         _stream(out), ctypes.byref(n)))
     return out, n.value
+
+
+def _crops_batch(name, images, n_rows, out, output_size):
+    """-> (hwc, channels, input dtype code, out) of a crops call: `out` defaults to a contiguous float32 [N,C,oH,oW]."""
+    import torch
+    n = len(images)
+    if n_rows != n:
+        raise ValueError(f"{name}: images and crops must have the same length")
+    hwc = bool(n) and _is_hwc(images[0])
+    if n:
+        C = images[0].shape[-1] if hwc else images[0].shape[0]
+    elif out is not None:
+        C = out.shape[1]
+    else:
+        raise ValueError(f"{name}: an empty batch needs `out`")
+    if out is None:
+        out = torch.empty((n, C, int(output_size[0]), int(output_size[1])), dtype=torch.float32, device=images[0].device)
+    return hwc, C, _dtype_code(images[0]) if n else F32, out
 
 
 def resize_crops(images, boxes, output_size, filter, out=None, hflip=None, scale=None, bias=None, align_corners=False, flags=FLAG_AUTO):
@@ -286,35 +288,22 @@ def resize_crops(images, boxes, output_size, filter, out=None, hflip=None, scale
     dtype (uint8 or float32); an image may repeat.  `boxes`: (top, left, height, width) per image.  `out` defaults to a
     contiguous float32 [N,C,oH,oW]; scale/bias (per channel, <= 4) apply v*scale[c] + bias[c] at the store.
     Returns (out, launches)."""
-    import torch
+    import numpy as np
     n = len(images)
     if len(boxes) != n or (hflip is not None and len(hflip) != n):
         raise ValueError("resize_crops: images, boxes and hflip must have the same length")
-    hwc = bool(n) and _is_hwc(images[0])
+    hwc, C, dtype, out = _crops_batch("resize_crops", images, n, out, output_size)
+    crops = np.zeros(n, np.dtype(Crop))
     if n:
-        C = images[0].shape[-1] if hwc else images[0].shape[0]
-    elif out is not None:
-        C = out.shape[1]
-    else:
-        raise ValueError("resize_crops: an empty batch needs `out`")
-    oH, oW = int(output_size[0]), int(output_size[1])
-    if out is None:
-        out = torch.empty((n, C, oH, oW), dtype=torch.float32, device=images[0].device)
-    arr = (ImageDesc * max(n, 1))()
-    crops = (Crop * max(n, 1))()
-    for i, t in enumerate(images):
-        if hwc:
-            arr[i] = ImageDesc(t.data_ptr(), t.shape[0], t.shape[1], t.stride(0), 1)
-        else:
-            arr[i] = ImageDesc(t.data_ptr(), t.shape[1], t.shape[2], t.stride(1), t.stride(0))
-        top, left, h, w = (int(v) for v in boxes[i])
-        crops[i] = Crop(top, left, h, w, int(bool(hflip[i])) if hflip is not None else 0)
+        crops["top"], crops["left"], crops["height"], crops["width"] = np.array(boxes, np.int64).reshape(n, 4).T
+        if hflip is not None:
+            crops["hflip"] = [bool(f) for f in hflip]
+    rows = image_descs(images, hwc)  # held until the call returns: only its address is passed
     e = _epilogue(scale, bias)
     k = ctypes.c_int32(0)
-    dtype = _dtype_code(images[0]) if n else F32
     do = desc(out)
-    check(lib().aa_resize_crops(arr, crops, n, dtype, C, int(hwc), ctypes.byref(do), _filter(filter), int(align_corners), flags,
-                                ctypes.byref(e), _stream(out), ctypes.byref(k)))
+    check(lib().aa_resize_crops(rows.ctypes.data, crops.ctypes.data, n, dtype, C, int(hwc), ctypes.byref(do), _filter(filter),
+                                int(align_corners), flags, ctypes.byref(e), _stream(out), ctypes.byref(k)))
     return out, k.value
 
 
@@ -343,45 +332,6 @@ def crop_ex_array(crops):
     return arr
 
 
-def launch_crops_ex(image_rows, crop_rows, dtype, channels, hwc, out, filter, scale=None, bias=None, align_corners=False,
-                    flags=FLAG_AUTO):
-    """aa_resize_crops_ex on descriptor arrays (image_descs / crop_ex_array, one row per crop) into `out`; -> launches."""
-    assert len(image_rows) == len(crop_rows) and image_rows.dtype == image_desc_dtype() and crop_rows.dtype == crop_ex_dtype()
-    assert image_rows.flags.c_contiguous and crop_rows.flags.c_contiguous
-    e = _epilogue(scale, bias)
-    k = ctypes.c_int32(0)
-    do = desc(out)
-    check(lib().aa_resize_crops_ex(image_rows.ctypes.data, crop_rows.ctypes.data, len(crop_rows), dtype, channels, int(hwc),
-                                   ctypes.byref(do), _filter(filter), int(align_corners), flags, ctypes.byref(e), _stream(out),
-                                   ctypes.byref(k)))
-    return k.value
-
-
-def resize_crops_ex(images, crops, output_size, filter, out=None, scale=None, bias=None, align_corners=False, flags=FLAG_AUTO):
-    """Batched resize-then-crop (aa_resize_crops_ex): out[i] = the output_size window at (crop_top, crop_left) of
-    resize(images[i][top:top+height, left:left+width]) to (resized_h, resized_w), flipped horizontally where bit 0 of flip is
-    set and vertically where bit 1 is.  `images` as in resize_crops; `crops`: one aa_crop_ex row per image, tuples
-    (top, left, height, width, resized_h, resized_w, crop_top, crop_left, flip), an [N, 9] integer array or a crop_ex_dtype
-    array.  `out` defaults to a contiguous float32 [N,C,oH,oW]; scale/bias as in resize_crops.  Returns (out, launches)."""
-    import torch
-    n = len(images)
-    rows = crop_ex_array(crops)
-    if len(rows) != n:
-        raise ValueError("resize_crops_ex: images and crops must have the same length")
-    hwc = bool(n) and _is_hwc(images[0])
-    if n:
-        C = images[0].shape[-1] if hwc else images[0].shape[0]
-    elif out is not None:
-        C = out.shape[1]
-    else:
-        raise ValueError("resize_crops_ex: an empty batch needs `out`")
-    oH, oW = int(output_size[0]), int(output_size[1])
-    if out is None:
-        out = torch.empty((n, C, oH, oW), dtype=torch.float32, device=images[0].device)
-    dtype = _dtype_code(images[0]) if n else F32
-    return out, launch_crops_ex(image_descs(images, hwc), rows, dtype, C, hwc, out, filter, scale, bias, align_corners, flags)
-
-
 def fill_struct(mode, value):
     """Fill of `mode` with `value`: a number for every channel or one number per channel (at most 4)."""
     f = Fill()
@@ -395,19 +345,37 @@ def fill_struct(mode, value):
     return f
 
 
-def launch_crops_pad(image_rows, crop_rows, dtype, channels, hwc, out, filter, fill_mode, fill_value, scale=None, bias=None,
-                     align_corners=False, flags=FLAG_AUTO):
-    """aa_resize_crops_pad on descriptor arrays (as launch_crops_ex) with the fill (fill_mode, fill_value); -> launches."""
+def launch_crops(image_rows, crop_rows, dtype, channels, hwc, out, filter, scale=None, bias=None, align_corners=False,
+                 flags=FLAG_AUTO, fill=None):
+    """The crops kernel on descriptor arrays (image_descs / crop_ex_array, one row per crop) into `out`; -> launches.
+    Without `fill` it calls aa_resize_crops_ex; with one, a (mode, value) pair or a Fill, aa_resize_crops_pad."""
     assert len(image_rows) == len(crop_rows) and image_rows.dtype == image_desc_dtype() and crop_rows.dtype == crop_ex_dtype()
     assert image_rows.flags.c_contiguous and crop_rows.flags.c_contiguous
-    e = _epilogue(scale, bias)
-    f = fill_struct(fill_mode, fill_value)
+    args = [image_rows.ctypes.data, crop_rows.ctypes.data, len(crop_rows), dtype, channels, int(hwc), ctypes.byref(desc(out)),
+            _filter(filter), int(align_corners), flags, ctypes.byref(_epilogue(scale, bias))]
+    if fill is None:
+        call = lib().aa_resize_crops_ex
+    else:
+        call = lib().aa_resize_crops_pad
+        args.append(ctypes.byref(fill if isinstance(fill, Fill) else fill_struct(*fill)))
     k = ctypes.c_int32(0)
-    do = desc(out)
-    check(lib().aa_resize_crops_pad(image_rows.ctypes.data, crop_rows.ctypes.data, len(crop_rows), dtype, channels, int(hwc),
-                                    ctypes.byref(do), _filter(filter), int(align_corners), flags, ctypes.byref(e),
-                                    ctypes.byref(f), _stream(out), ctypes.byref(k)))
+    check(call(*args, _stream(out), ctypes.byref(k)))
     return k.value
+
+
+def _resize_crops(name, images, crops, output_size, filter, out, scale, bias, align_corners, flags, fill):
+    rows = crop_ex_array(crops)
+    hwc, C, dtype, out = _crops_batch(name, images, len(rows), out, output_size)
+    return out, launch_crops(image_descs(images, hwc), rows, dtype, C, hwc, out, filter, scale, bias, align_corners, flags, fill)
+
+
+def resize_crops_ex(images, crops, output_size, filter, out=None, scale=None, bias=None, align_corners=False, flags=FLAG_AUTO):
+    """Batched resize-then-crop (aa_resize_crops_ex): out[i] = the output_size window at (crop_top, crop_left) of
+    resize(images[i][top:top+height, left:left+width]) to (resized_h, resized_w), flipped horizontally where bit 0 of flip is
+    set and vertically where bit 1 is.  `images` as in resize_crops; `crops`: one aa_crop_ex row per image, tuples
+    (top, left, height, width, resized_h, resized_w, crop_top, crop_left, flip), an [N, 9] integer array or a crop_ex_dtype
+    array.  `out` defaults to a contiguous float32 [N,C,oH,oW]; scale/bias as in resize_crops.  Returns (out, launches)."""
+    return _resize_crops("resize_crops_ex", images, crops, output_size, filter, out, scale, bias, align_corners, flags, None)
 
 
 def resize_crops_pad(images, crops, output_size, filter, fill=0.0, fill_mode=FILL_INPUT, out=None, scale=None, bias=None,
@@ -416,24 +384,8 @@ def resize_crops_pad(images, crops, output_size, filter, fill=0.0, fill_mode=FIL
     negative crop_top / crop_left, or past its end); outputs there store `fill` (one number, or one per channel), as a
     pixel value of the input (FILL_INPUT) or as it is (FILL_OUTPUT).  Arguments as in resize_crops_ex.
     Returns (out, launches)."""
-    import torch
-    n = len(images)
-    rows = crop_ex_array(crops)
-    if len(rows) != n:
-        raise ValueError("resize_crops_pad: images and crops must have the same length")
-    hwc = bool(n) and _is_hwc(images[0])
-    if n:
-        C = images[0].shape[-1] if hwc else images[0].shape[0]
-    elif out is not None:
-        C = out.shape[1]
-    else:
-        raise ValueError("resize_crops_pad: an empty batch needs `out`")
-    oH, oW = int(output_size[0]), int(output_size[1])
-    if out is None:
-        out = torch.empty((n, C, oH, oW), dtype=torch.float32, device=images[0].device)
-    dtype = _dtype_code(images[0]) if n else F32
-    return out, launch_crops_pad(image_descs(images, hwc), rows, dtype, C, hwc, out, filter, fill_mode, fill, scale, bias,
-                                 align_corners, flags)
+    return _resize_crops("resize_crops_pad", images, crops, output_size, filter, out, scale, bias, align_corners, flags,
+                         (fill_mode, fill))
 
 
 def resize_backward(grad_out, input_size, filter, align_corners=False, nonaa=False, flags=FLAG_AUTO, scales=None, out=None):

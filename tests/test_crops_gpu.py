@@ -8,7 +8,7 @@ import random
 
 import pytest
 
-FILL_NAN = float("nan")
+from crops_common import BIAS, BOXES, FILL_NAN, OUTS, SCALE, _assert_same_bits, _images, _reference, _view
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -85,69 +85,12 @@ def test_crops_valid_arguments_need_a_device():
 
 
 # ---------------------------------------------------------------------------------------------------------------------
-# GPU: reference = aa_resize_forward_ex on the crop's view with FLAG_FORCE_GENERAL
+# GPU: reference = aa_resize_forward_ex on the crop's view with FLAG_FORCE_GENERAL (crops_common._reference)
 # ---------------------------------------------------------------------------------------------------------------------
-def _view(img, hwc, box):
-    top, left, h, w = box
-    if hwc:
-        return img[top:top + h, left:left + w, :].permute(2, 0, 1).unsqueeze(0)
-    return img[:, top:top + h, left:left + w].unsqueeze(0)
-
-
-def _reference(capi, images, boxes, hflip, osize, filt, align, out_dtype, scale=None, bias=None, flags=0):
-    import torch
-    hwc = capi._is_hwc(images[0])
-    C = images[0].shape[-1] if hwc else images[0].shape[0]
-    outs = []
-    for img, box, f in zip(images, boxes, hflip):
-        o = torch.empty((1, C) + tuple(osize), dtype=out_dtype, device=img.device)
-        capi.resize_forward_ex(_view(img, hwc, box), osize, filt, o, scale, bias, align, flags | capi.FLAG_FORCE_GENERAL)
-        outs.append(o.flip(-1) if f else o)
-    return torch.cat(outs)
-
-
-def _bits(t):
-    import torch
-    return t.view({4: torch.int32, 2: torch.int16, 1: torch.uint8}[t.element_size()])
-
-
-def _assert_same_bits(got, want, what):
-    import torch
-    g, w = _bits(got.contiguous()), _bits(want.contiguous())
-    if not torch.equal(g, w):
-        bad = (g != w).nonzero()
-        raise AssertionError(f"{what}: {bad.shape[0]} of {g.numel()} outputs differ, first at {bad[0].tolist()}: "
-                             f"{got[tuple(bad[0])].item()} vs {want[tuple(bad[0])].item()}")
-
-
-def _images(kind, C, dev, seed):
-    """Two images per kind: 300x400 and a 1080p frame, as HWC or planar tensors."""
-    import torch
-    g = torch.Generator(device=dev).manual_seed(seed)
-    hwc = kind.endswith("hwc")
-    imgs = []
-    for H, W in ((300, 400), (1080, 1920)):
-        shape = (H, W, C) if hwc else (C, H, W)
-        if kind.startswith("u8"):
-            imgs.append(torch.randint(0, 256, shape, generator=g, device=dev, dtype=torch.uint8))
-        else:
-            imgs.append(torch.rand(shape, generator=g, device=dev) * 255)
-    return imgs
-
-
-# (image index, box): 4x upsampling, about 1x, 0.75x from the top-left corner, a full 1080p frame to 224^2, 1-pixel-high and
-# 1-pixel-wide boxes (the latter on the right edge), the bottom-right corner of both images, the same image several times
-BOXES = [(0, (100, 120, 56, 56)), (0, (10, 20, 224, 230)), (0, (0, 0, 299, 299)), (1, (0, 0, 1080, 1920)),
-         (0, (150, 30, 1, 200)), (0, (40, 399, 150, 1)), (0, (180, 200, 120, 200)), (0, (5, 5, 290, 390)),
-         (1, (500, 900, 580, 1020))]
-OUTS = {  # name: (torch dtype name, flags, affine)
-    "f32": ("float32", 0, False),
-    "u8": ("uint8", 0, False),
-    "u8_round": ("uint8", "FLAG_ROUND_NEAREST", False),
-    "f16_affine": ("float16", 0, True),
-    "bf16_affine": ("bfloat16", 0, True),
-}
-SCALE, BIAS = [0.0174, -0.031, 2.5, 1.0 / 255], [-2.1, 0.75, -300.0, 0.5]
+def _as_ex(boxes, hflip, osize):
+    """aa_resize_crops crops as aa_crop_ex rows for _reference: each box resized to the output size, the window at the
+    origin, the horizontal flip bit from hflip."""
+    return [tuple(b) + tuple(osize) + (0, 0, int(bool(f))) for b, f in zip(boxes, hflip)]
 
 
 @pytest.mark.gpu
@@ -169,7 +112,8 @@ def test_crops_parity_matrix(cuda, filt, align, kind, out_kind):
         out = torch.empty((len(boxes), C, 224, 224), dtype=out_dtype, device=cuda)
         got, launches = capi.resize_crops(images, boxes, (224, 224), filt, out=out, hflip=hflip, scale=scale, bias=bias,
                                           align_corners=bool(align), flags=flags)
-        want = _reference(capi, images, boxes, hflip, (224, 224), filt, bool(align), out_dtype, scale, bias, flags)
+        want = _reference(capi, images, _as_ex(boxes, hflip, (224, 224)), (224, 224), filt, bool(align), out_dtype, scale,
+                          bias, flags)
         assert launches == 1
         _assert_same_bits(got, want, f"{kind} C={C} {filt} align={align} {out_kind}")
 
@@ -184,7 +128,7 @@ def test_crops_hwc_into_channels_last_output(cuda):
     hflip = [i % 3 == 0 for i in range(len(boxes))]
     out = torch.empty((len(boxes), 3, 100, 130), device=cuda, memory_format=torch.channels_last)
     got, _ = capi.resize_crops(images, boxes, (100, 130), "bicubic", out=out, hflip=hflip)
-    want = _reference(capi, images, boxes, hflip, (100, 130), "bicubic", False, torch.float32)
+    want = _reference(capi, images, _as_ex(boxes, hflip, (100, 130)), (100, 130), "bicubic", False, torch.float32)
     _assert_same_bits(got, want, "HWC -> channels_last")
 
 
@@ -209,7 +153,7 @@ def test_crops_more_than_one_launch(cuda):
     capi.launch_count(reset=True)
     got, launches = capi.resize_crops(images, boxes, (20, 28), "bilinear", hflip=hflip)
     assert launches == 3 and capi.launch_count(reset=True) == 3
-    want = _reference(capi, images, boxes, hflip, (20, 28), "bilinear", False, torch.float32)
+    want = _reference(capi, images, _as_ex(boxes, hflip, (20, 28)), (20, 28), "bilinear", False, torch.float32)
     _assert_same_bits(got, want, "1100 crops")
 
 
@@ -274,7 +218,8 @@ def test_crops_read_only_inside_the_boxes(cuda, hwc):
         out = parent[1:, 1:, 2:66, 1:73]
         got, _ = capi.resize_crops(imgs, boxes, (64, 72), "bicubic", out=out, hflip=hflip,
                                    scale=[1.0] * C if dt == torch.float16 else None)
-        want = _reference(capi, imgs, boxes, hflip, (64, 72), "bicubic", False, dt, [1.0] * C if dt == torch.float16 else None)
+        want = _reference(capi, imgs, _as_ex(boxes, hflip, (64, 72)), (64, 72), "bicubic", False, dt,
+                          [1.0] * C if dt == torch.float16 else None)
         _assert_same_bits(out, want, f"padded view {dt}")
         mask = torch.ones(parent.shape, dtype=torch.bool, device=cuda)
         mask[1:, 1:, 2:66, 1:73] = False
@@ -303,7 +248,7 @@ def test_crops_nonfinite_placement(cuda, hwc):
     for mode in ("box", "bilinear", "bicubic"):
         for osize in ((224, 224), (17, 23)):
             got, n = capi.resize_crops([img] * len(boxes), boxes, osize, mode, hflip=hflip)
-            want = _reference(capi, [img] * len(boxes), boxes, hflip, osize, mode, False, torch.float32)
+            want = _reference(capi, [img] * len(boxes), _as_ex(boxes, hflip, osize), osize, mode, False, torch.float32)
             assert n == 1
             assert torch.equal(torch.isnan(got), torch.isnan(want)), (mode, osize)
             assert bool(torch.isnan(got).any() or torch.isinf(got).any()), (mode, osize)
@@ -366,7 +311,8 @@ def test_crops_64bit_offsets(cuda):
         v = img[b[0]:b[0] + b[2], b[1]:b[1] + b[3]]
         v.copy_(torch.randint(0, 256, v.shape, generator=g, device=cuda, dtype=torch.uint8))
     got, _ = capi.resize_crops([img] * 3, boxes, (224, 224), "bicubic", hflip=[True, False, False])
-    want = _reference(capi, [img] * 3, boxes, [True, False, False], (224, 224), "bicubic", False, torch.float32)
+    want = _reference(capi, [img] * 3, _as_ex(boxes, [True, False, False], (224, 224)), (224, 224), "bicubic", False,
+                      torch.float32)
     _assert_same_bits(got, want, "64-bit offsets")
     del img
     torch.cuda.empty_cache()
@@ -392,11 +338,12 @@ def test_resized_crops_python_api(cuda):
                                 scale=[1.0 / (255.0 * s) for s in std], bias=[-m / s for m, s in zip(mean, std)])
     assert n == 1
     _assert_same_bits(y, want, "resized_crops fp16")
-    ref = _reference(capi, imgs, boxes, hflip, (224, 224), "bilinear", False, torch.float16,
+    ref = _reference(capi, imgs, _as_ex(boxes, hflip, (224, 224)), (224, 224), "bilinear", False, torch.float16,
                      [1.0 / (255.0 * s) for s in std], [-m / s for m, s in zip(mean, std)])
     _assert_same_bits(y, ref, "resized_crops vs general")
     y8 = aa.resized_crops(imgs, boxes, (200, 180), mode="bicubic", hflip=hflip, out_dtype=torch.uint8)
-    want8 = _reference(capi, imgs, boxes, hflip, (200, 180), "bicubic", False, torch.uint8, flags=capi.FLAG_ROUND_NEAREST)
+    want8 = _reference(capi, imgs, _as_ex(boxes, hflip, (200, 180)), (200, 180), "bicubic", False, torch.uint8,
+                       flags=capi.FLAG_ROUND_NEAREST)
     _assert_same_bits(y8, want8, "resized_crops uint8")
     # one 4-D tensor, contiguous and channels_last, float32 output
     x = torch.rand((4, 3, 120, 160), generator=g, device=cuda) * 255
@@ -404,5 +351,6 @@ def test_resized_crops_python_api(cuda):
     for xx in (x, x.contiguous(memory_format=torch.channels_last)):
         y4 = aa.resized_crops(xx, b4, (64, 64), mode="bicubic", hflip=[False, True, False, True])
         assert y4.dtype == torch.float32 and y4.is_contiguous()
-        w4 = _reference(capi, list(x.unbind(0)), b4, [False, True, False, True], (64, 64), "bicubic", False, torch.float32)
+        w4 = _reference(capi, list(x.unbind(0)), _as_ex(b4, [False, True, False, True], (64, 64)), (64, 64), "bicubic", False,
+                        torch.float32)
         _assert_same_bits(y4, w4, "4-D input")

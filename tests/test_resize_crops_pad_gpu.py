@@ -10,7 +10,7 @@ import random
 
 import pytest
 
-from test_resize_crops_ex_gpu import BIAS, OK, OUTS, SCALE, WINDOWS, _assert_same_bits, _host_args, _images, _view
+from crops_common import BIAS, OK, OUTS, SCALE, WINDOWS, _assert_same_bits, _host_args, _images, _reference, _view
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -161,38 +161,6 @@ def test_resize_pad_batch_layout():
 FILL = [114.6, -0.0, 300.5, 7.3]  # a u8 clamp and rounding, a negative zero, a value no half-precision type holds
 
 
-def _fill_value(capi, C, fill, mode, out_dtype, scale, bias, flags, dev):
-    """[C] tensor: the 1x1 resize of a [1, C, 1, 1] float32 tensor holding the fill."""
-    import torch
-    x = torch.tensor(fill[:C] if len(fill) >= C else fill * C, dtype=torch.float32, device=dev).view(1, C, 1, 1)
-    o = torch.empty((1, C, 1, 1), dtype=out_dtype, device=dev)
-    if mode == capi.FILL_OUTPUT:
-        scale = bias = None
-    capi.resize_forward_ex(x, (1, 1), "bilinear", o, scale, bias, False, flags | capi.FLAG_FORCE_GENERAL)
-    return o.view(C)
-
-
-def _pad_reference(capi, images, crops, osize, filt, align, out_dtype, fill, mode, scale=None, bias=None, flags=0):
-    import torch
-    hwc = capi._is_hwc(images[0])
-    C = images[0].shape[-1] if hwc else images[0].shape[0]
-    oH, oW = osize
-    fv = _fill_value(capi, C, fill, mode, out_dtype, scale, bias, flags, images[0].device)
-    outs = []
-    for img, c in zip(images, crops):
-        top, left, h, w, rh, rw, ct, cl, flip = (int(v) for v in c)
-        win = fv.view(1, C, 1, 1).expand(1, C, oH, oW).clone()
-        y0, y1, x0, x1 = max(ct, 0), min(ct + oH, rh), max(cl, 0), min(cl + oW, rw)
-        if y0 < y1 and x0 < x1:
-            r = torch.empty((1, C, rh, rw), dtype=out_dtype, device=img.device)
-            capi.resize_forward_ex(_view(img, hwc, (top, left, h, w)), (rh, rw), filt, r, scale, bias, align,
-                                   flags | capi.FLAG_FORCE_GENERAL)
-            win[:, :, y0 - ct:y1 - ct, x0 - cl:x1 - cl] = r[:, :, y0:y1, x0:x1]
-        dims = ([-1] if flip & 1 else []) + ([-2] if flip & 2 else [])
-        outs.append(win.flip(dims) if dims else win)
-    return torch.cat(outs)
-
-
 # output size -> [(image index, aa_crop_ex without flip)]; image 0 is 300x400, image 1 1080x1920
 PAD_WINDOWS = {
     (48, 64): [
@@ -249,7 +217,8 @@ def test_crops_pad_parity_matrix(cuda, filt, align, kind, out_kind, fill_mode):
             out = torch.empty((len(crops), C) + osize, dtype=out_dtype, device=cuda)
             got, launches = capi.resize_crops_pad(images, crops, osize, filt, FILL[:C], mode, out=out, scale=scale, bias=bias,
                                                   align_corners=bool(align), flags=flags)
-            want = _pad_reference(capi, images, crops, osize, filt, bool(align), out_dtype, FILL[:C], mode, scale, bias, flags)
+            want = _reference(capi, images, crops, osize, filt, bool(align), out_dtype, scale, bias, flags, fill=FILL[:C],
+                              fill_mode=mode)
             assert launches == 1
             _assert_same_bits(got, want, f"{kind} C={C} {filt} align={align} {out_kind} {fill_mode} {osize}")
 
@@ -378,8 +347,8 @@ def test_padded_helpers_bitwise(cuda):
                           dtype=torch.uint8) for _ in range(9)]
     y = aa.resize_center_crop(imgs, 200, 256, mean=mean, std=std, pad=True)
     rows = aa._eval_crops([t.shape[:2] for t in imgs], 200, 256, "center", pad=True).reshape(-1)
-    want = _pad_reference(capi, imgs, [tuple(int(v) for v in r) for r in rows], (256, 256), "bilinear", False, torch.float16,
-                          [0.0], capi.FILL_INPUT, scale, bias)
+    want = _reference(capi, imgs, [tuple(int(v) for v in r) for r in rows], (256, 256), "bilinear", False, torch.float16,
+                      scale, bias, fill=[0.0], fill_mode=capi.FILL_INPUT)
     _assert_same_bits(y, want, "resize_center_crop(pad=True)")
     # nothing to pad: the same bits as pad=False
     _assert_same_bits(aa.resize_center_crop(imgs, 256, 150, mean=mean, std=std, pad=True),
@@ -389,8 +358,8 @@ def test_padded_helpers_bitwise(cuda):
             batch, place = aa.resize_pad_batch(imgs, 224, max_size=300, align=align, mean=mean, std=std, **kw)
             crops = [(0, 0, t.shape[0], t.shape[1], h, w, -top, -left, 0) for t, (top, left, h, w) in zip(imgs, place.tolist())]
             value = list(kw.get("fill", (kw.get("pad_value", 0.0),)))
-            want = _pad_reference(capi, imgs, crops, tuple(batch.shape[-2:]), "bilinear", False, torch.float16, value * 3
-                                  if len(value) == 1 else value, mode, scale, bias)
+            want = _reference(capi, imgs, crops, tuple(batch.shape[-2:]), "bilinear", False, torch.float16, scale, bias,
+                              fill=value * 3 if len(value) == 1 else value, fill_mode=mode)
             _assert_same_bits(batch, want, f"resize_pad_batch {kw} {align}")
 
 
@@ -419,8 +388,8 @@ def test_crops_pad_read_inside_boxes_store_inside_output(cuda, hwc):
         imgs = [image(float("nan"), torch.float32, c) for c in crops]
         got, _ = capi.resize_crops_pad(imgs, crops, (64, 72), mode, [1.0, 2.0, 3.0], capi.FILL_INPUT)
         assert bool(torch.isfinite(got).all()), mode
-        _assert_same_bits(got, _pad_reference(capi, imgs, crops, (64, 72), mode, False, torch.float32, [1.0, 2.0, 3.0],
-                                              capi.FILL_INPUT), f"NaN parents {mode}")
+        _assert_same_bits(got, _reference(capi, imgs, crops, (64, 72), mode, False, torch.float32, fill=[1.0, 2.0, 3.0],
+                                          fill_mode=capi.FILL_INPUT), f"NaN parents {mode}")
         # uint8: canary 0 and 255 outside the boxes give the same bits
         g.manual_seed(12)
         a = [image(0, torch.uint8, c) for c in crops]
@@ -437,8 +406,8 @@ def test_crops_pad_read_inside_boxes_store_inside_output(cuda, hwc):
         scale = [1.0] * C if dt == torch.float16 else None
         for mode in (capi.FILL_INPUT, capi.FILL_OUTPUT):
             capi.resize_crops_pad(imgs, crops, (64, 72), "bicubic", 5.0, mode, out=out, scale=scale)
-            _assert_same_bits(out, _pad_reference(capi, imgs, crops, (64, 72), "bicubic", False, dt, [5.0] * 3, mode, scale),
-                              f"padded view {dt}")
+            _assert_same_bits(out, _reference(capi, imgs, crops, (64, 72), "bicubic", False, dt, scale, fill=[5.0] * 3,
+                                              fill_mode=mode), f"padded view {dt}")
             mask = torch.ones(parent.shape, dtype=torch.bool, device=cuda)
             mask[1:, 1:, 2:66, 1:73] = False
             outside = parent[mask]
@@ -471,8 +440,8 @@ def test_crops_pad_nonfinite_placement(cuda, hwc):
                     crops.append((0, 0, 200, 260, rh, rw, ct, cl, (j + k) % 4))
             for fill in (0.0, float("nan")):
                 got, n = capi.resize_crops_pad([img] * len(crops), crops, osize, mode, fill, capi.FILL_INPUT)
-                want = _pad_reference(capi, [img] * len(crops), crops, osize, mode, False, torch.float32, [fill] * 3,
-                                      capi.FILL_INPUT)
+                want = _reference(capi, [img] * len(crops), crops, osize, mode, False, torch.float32, fill=[fill] * 3,
+                                  fill_mode=capi.FILL_INPUT)
                 assert n == 1
                 assert torch.equal(torch.isnan(got), torch.isnan(want)), (mode, osize, fill)
                 assert fill != 0.0 or not bool(torch.isfinite(got).all()), (mode, osize)
@@ -496,8 +465,8 @@ def test_crops_pad_launches_and_graph_capture(cuda):
     assert capi.launch_count(reset=True) == 3
     assert batch.shape == (1100, 3, 48, 48) and batch.dtype == torch.float32 and batch.is_contiguous()
     crops = [(0, 0, t.shape[0], t.shape[1], h, w, -top, -left, 0) for t, (top, left, h, w) in zip(imgs, place.tolist())]
-    _assert_same_bits(batch, _pad_reference(capi, imgs, crops, (48, 48), "bicubic", False, torch.float32, [114.0] * 3,
-                                            capi.FILL_INPUT), "1100 crops")
+    _assert_same_bits(batch, _reference(capi, imgs, crops, (48, 48), "bicubic", False, torch.float32, fill=[114.0] * 3,
+                                        fill_mode=capi.FILL_INPUT), "1100 crops")
     # float input: one launch (no drain); capture once, replay on new pixel data
     imgs = [torch.rand((rnd.randint(64, 200), rnd.randint(64, 200), 3), generator=g, device=cuda) * 255 for _ in range(512)]
     crops = []
@@ -513,8 +482,8 @@ def test_crops_pad_launches_and_graph_capture(cuda):
     capi.launch_count(reset=True)
     _, n = capi.resize_crops_pad(imgs, crops, (56, 56), "bilinear", [3, 4, 5], capi.FILL_OUTPUT, out=out, **kw)
     assert n == 1 and capi.launch_count(reset=True) == 1
-    _assert_same_bits(out, _pad_reference(capi, imgs, crops, (56, 56), "bilinear", False, torch.float16, [3, 4, 5],
-                                          capi.FILL_OUTPUT, **kw), "512 crops")
+    _assert_same_bits(out, _reference(capi, imgs, crops, (56, 56), "bilinear", False, torch.float16, fill=[3, 4, 5],
+                                      fill_mode=capi.FILL_OUTPUT, **kw), "512 crops")
     torch.cuda.synchronize()
     graph = torch.cuda.CUDAGraph()
     s = torch.cuda.Stream()
@@ -552,8 +521,8 @@ def test_crops_pad_64bit_offsets(cuda):
         v = img[c[0]:c[0] + c[2], c[1]:c[1] + c[3]]
         v.copy_(torch.randint(0, 256, v.shape, generator=g, device=cuda, dtype=torch.uint8))
     got, _ = capi.resize_crops_pad([img] * len(crops), crops, (150, 120), "bicubic", 50.0, capi.FILL_INPUT)
-    want = _pad_reference(capi, [img] * len(crops), crops, (150, 120), "bicubic", False, torch.float32, [50.0] * 3,
-                          capi.FILL_INPUT)
+    want = _reference(capi, [img] * len(crops), crops, (150, 120), "bicubic", False, torch.float32, fill=[50.0] * 3,
+                      fill_mode=capi.FILL_INPUT)
     _assert_same_bits(got, want, "64-bit offsets")
     del img
     torch.cuda.empty_cache()
